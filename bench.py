@@ -67,7 +67,16 @@ def parse():
     p.add_argument("--ncu", action="store_true",
                    help="profiling run: 1 warm-up + 1 step between cudaProfilerStart/Stop, no e2e / CPU legs "
                         "(use with ncu --profile-from-start off; numbers printed under ncu are not bench values)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write what the last of them computed as DIR/<name>.npy: its loss, "
+                        "a fixed seeded sample of the updated parameters and of their gradients, and the BN "
+                        "buffers (~34 MB); the inputs depend only on the arguments, so two builds can be compared")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.ncu):
+        p.error("--dump-outputs needs the timed CUDA path (--impl ours, without --ncu)")
+    return args
 
 
 def peaks():
@@ -224,6 +233,30 @@ def cpu_baseline(args):
 
 
 # ------------------------------------------------------------------------------------------ CUDA arm
+DUMP_SAMPLE = 1 << 22  # elements kept of the parameter and gradient vectors: 2 x 16 MB of float32
+
+
+def dump_outputs(path, model, loss):
+    """What one training step hands its caller, as float32 / float64 .npy files under `path`:
+    loss.npy        the total loss the step returned
+    parameters.npy  the parameters after the Adam step  } all parameters flattened in named_parameters() order,
+    gradients.npy   the gradients that step applied     } then the same fixed seeded sample of DUMP_SAMPLE elements
+                    (zero for a parameter the step gave no gradient)
+    buffers.npy     every buffer (BN running statistics, batch counters) flattened in named_buffers() order, float64"""
+    os.makedirs(path, exist_ok=True)
+    params = [p for _, p in model.named_parameters()]
+    n = sum(p.numel() for p in params)
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(DUMP_SAMPLE, n), replace=False))
+    idx = torch.from_numpy(idx).to(params[0].device)
+    out = {"loss": loss.detach().float().cpu().numpy(),
+           "parameters": torch.cat([p.detach().reshape(-1) for p in params])[idx].float().cpu().numpy(),
+           "gradients": torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1)
+                                   for p in params])[idx].float().cpu().numpy(),
+           "buffers": torch.cat([b.detach().reshape(-1).double() for _, b in model.named_buffers()]).cpu().numpy()}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch.distributed as dist
     from lidog_b200 import cabi
@@ -312,10 +345,12 @@ def run_ours(args):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms)
 
+    last = {}
+
     def resident_step():
         if args.empty_cache:
             torch.cuda.empty_cache()
-        trainer.training_step(dev_pts, dev_lab)
+        last["loss"] = trainer.training_step(dev_pts, dev_lab)
 
     def e2e_step():
         if args.empty_cache:
@@ -343,6 +378,8 @@ def run_ours(args):
     clocks = sampler.stop() if sampler else None
     ms_per_step = total_ms / args.steps
     value = world * args.batch / (ms_per_step / 1e3)
+    if args.dump_outputs and rank == 0:  # before the passes below train the model further
+        dump_outputs(args.dump_outputs, net, last["loss"])
 
     # ---- separate passes (untimed for the headline): launch census, pair census, per-launch kernel times
     cabi.counting(True)

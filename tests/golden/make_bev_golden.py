@@ -1,7 +1,7 @@
 """Generate golden vectors for the BEV projection by running the REFERENCE's own
 `MinkUNetBaseBEV.sparse2super` (utils/models/minkunet_bev.py:169-230) on CPU.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the reference at oracle/_ref/ (tests/refharness.py):
     python tests/golden/make_bev_golden.py
 The reference imports MinkowskiEngine at module scope; an empty stand-in module
 satisfies the import (sparse2super itself is plain torch).  torch is pinned to
@@ -16,8 +16,8 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-REF = "/root/reference"
 OUT = os.path.dirname(os.path.abspath(__file__))
+REF = os.path.join(os.path.dirname(os.path.dirname(OUT)), "oracle", "_ref")
 
 
 def _import_reference_model():

@@ -1,5 +1,5 @@
 """Golden vectors for the losses, the BEV label image and the dataset-side filters, produced by the REFERENCE's own
-code (run in the build container only -- needs /root/reference):
+code (needs a checkout of the reference at oracle/_ref/, tests/refharness.py):
 
     python tests/golden/make_reference_golden.py        -> tests/golden/reference_step_products.npz
 
@@ -7,7 +7,7 @@ code (run in the build container only -- needs /root/reference):
                                                 loss value and d loss / d logits
   * utils/datasets/semantickitti_bev.py:433-464 PC2ImgConverter.getBEVImageNew, arguments prepared as at :137-153,:244-249
   * utils/datasets/semantickitti_bev.py:155-172 filter_bounds;  utils/datasets/dataset.py:58-72 random_sample (seeded)
-The GPU box has no /root/reference: tests/test_golden_reference.py replays these inputs through
+The reference is not part of this repository: tests/test_golden_reference.py replays these inputs through
 lidog_b200/lidog/{losses,step,datapath}.py on the CPU (everywhere) and on the device (-m gpu)."""
 import os
 import sys
@@ -19,13 +19,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 
 from tests import refharness as rh  # noqa: E402
+from tests.golden.inputs import REGENERATED, seeded_inputs, sha256  # noqa: E402
 from tests.test_reference_unchanged import _reference_class  # noqa: E402
 
 
 def main():
     from oracle import me_cpu
-    from oracle import voxel as ov
-    from lidog_b200.lidog import synth
+    inputs = seeded_inputs()
     out = {}
     with rh.reference(me_cpu):
         ref = rh.load_file("utils/losses/losses.py", "losses")
@@ -43,16 +43,13 @@ def main():
                 v.backward()
                 out[f"loss{C}_{name}"], out[f"loss{C}_{name}_grad"] = np.float64(v.item()), x.grad.numpy()
     Conv = _reference_class("utils/datasets/semantickitti_bev.py", "PC2ImgConverter")
-    for tag, seed, shape, bound, img in (("kitti", 5, "kitti", 50.0, 167), ("nusc", 3, "nuscenes", 30.0, 100)):
-        pts, lab = synth.make_scan(seed, shape)
-        keep = (np.abs(pts[:, 0]) < 35) & (np.abs(pts[:, 1]) < 35)
-        pts, lab = pts[keep][::3], lab[keep][::3]
-        q, _, colab, vidx, _ = ov.sparse_quantize(pts, np.ones((len(pts), 1), np.float32), lab, -1, True, True, False, 0.05)
+    for tag, bound, img in (("kitti", 50.0, 167), ("nusc", 30.0, 100)):
+        q, colab = inputs[f"bev_{tag}_coords"], inputs[f"bev_{tag}_colabels"]
         bounds = [[-bound, bound], [-bound, bound], [-10, 8]]
         conv = Conv(imgChannel=1, xRange=bounds[0], yRange=bounds[1], zRange=bounds[2], xGridSize=2 * bound / img,
                     yGridSize=2 * bound / img, zGridSize=0.3)
         bl, _ = conv.getBEVImageNew((q * 0.05).astype(np.float32), colab)
-        out[f"bev_{tag}_coords"], out[f"bev_{tag}_colabels"] = q.astype(np.int32), colab.astype(np.int32)
+        out[f"bev_{tag}_coords"], out[f"bev_{tag}_colabels"] = q, colab
         out[f"bev_{tag}_image"], out[f"bev_{tag}_bound_img"] = bl.astype(np.int32), np.array([bound, img])
     # dataset-side filter + augmentation: plain numpy on `self.*` attributes / module-level scipy
     import ast
@@ -63,9 +60,7 @@ def main():
 
     class Self:
         grid_bounds = [[-60, 60], [-60, 60], [-10, 8]]  # semantickitti_bev.py:137
-    rng = np.random.default_rng(11)
-    cloud = np.concatenate([rng.uniform(-70, 70, (4000, 2)), rng.uniform(-12, 10, (4000, 1))], 1).astype(np.float32)
-    cloud[:200, :2] = rng.uniform(-3.5, 3.5, (200, 2)).astype(np.float32)  # around the ego box
+    cloud = inputs["filter_points"]
     out["filter_points"], out["filter_keep"] = cloud, np.asarray(ns["filter_bounds"](Self(), cloud))
     from scipy.linalg import expm, norm
     asrc = open(rh.REF + "/utils/common/augmentation.py").read()
@@ -74,10 +69,12 @@ def main():
         if isinstance(node, ast.ClassDef) and node.name in ("RandomRotation", "RandomScale"):
             exec(compile(ast.Module(body=[node], type_ignores=[]), "augmentation.py", "exec"), ans)
     np.random.seed(1234)  # configs/lidog/single/semantickitti.yaml:32
-    pts32 = rng.uniform(-40, 40, (3000, 3)).astype(np.float32)
+    pts32 = inputs["aug_points"]
     aug = ans["RandomScale"](0.95, 1.05)(ans["RandomRotation"]()(pts32.copy()))  # order of train_lidog's Compose
     out["aug_points"], out["aug_result"] = pts32, np.asarray(aug)
     assert out["aug_result"].dtype == np.float64  # float32 @ float64: what sparse_quantize then receives
+    out = {(k + "_sha256" if k in REGENERATED else k): (np.array(sha256(v)) if k in REGENERATED else v)
+           for k, v in out.items()}
     np.savez_compressed(os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_step_products.npz"), **out)
     print({k: getattr(v, "shape", v) for k, v in out.items()})
 

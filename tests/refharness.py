@@ -1,7 +1,8 @@
 """Harness (test infrastructure only) for running the reference's OWN Python files unchanged.
 
-/root/reference exists in the build container but not on the GPU box, so these helpers are used by CPU tests that skip
-when it is absent, and by tests/golden/make_*_golden.py, which commit what the reference computes as fixtures.
+The reference (the original LiDOG sources) is not part of this repository: put a checkout of it at oracle/_ref/
+(git-ignored) to run them.  These helpers are used by CPU tests that skip when it is absent, and by
+tests/golden/make_*_golden.py, which commit what the reference computes as fixtures.
 
 The reference's files import `MinkowskiEngine`, `pytorch_lightning` and `torchmetrics` (SURVEY.md Appendix D).  The
 first is bound to the module under test (the CPU oracle shim or the CUDA product), the other two to the minimal
@@ -18,7 +19,7 @@ import types
 
 import torch
 
-REF = "/root/reference"
+REF = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
 
 
 def reference_available() -> bool:

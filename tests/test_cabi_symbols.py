@@ -95,25 +95,25 @@ def test_no_cpu_fallback():
 
 def test_model_state_dict_matches_reference_names():
     """Parameter names/shapes of the table-driven model equal the reference class's (checked against
-    the unchanged reference file when /root/reference is present, else against the expected counts)."""
+    the unchanged reference file when a checkout of it is at oracle/_ref/, else against the expected counts)."""
     from lidog_b200.lidog.model import MinkUNet34BEV
     import MinkowskiEngine as ME
+    from tests import refharness as rh
     m = MinkUNet34BEV(1, 7)
     sd = {k: tuple(v.shape) for k, v in m.state_dict().items()}
     assert len(sd) == 388 and sum(p.numel() for p in m.parameters()) == 38_660_622
     assert sd["conv0p1s1.kernel"] == (125, 1, 32) and sd["final.kernel"] == (96, 7) and sd["final.bias"] == (1, 7)
     assert sd["block5.0.downsample.0.kernel"] == (384, 256) and sd["convtr4p16s2.kernel"] == (8, 256, 256)
     assert "encoders2d.block8.down1.maxpool_conv.0.double_conv.0.weight" in sd
-    ref_file = "/root/reference/utils/models/minkunet_bev.py"
-    if os.path.exists(ref_file):
+    if rh.reference_available():
         import sys
-        sys.path.insert(0, "/root/reference")
+        sys.path.insert(0, rh.REF)
         try:
             import utils.models.minkunet_bev as ref  # the UNCHANGED reference file on the drop-in package
             r = ref.MinkUNet34BEV(1, 7, 3)
             assert {k: tuple(v.shape) for k, v in r.state_dict().items()} == sd
         finally:
-            sys.path.remove("/root/reference")
+            sys.path.remove(rh.REF)
 
 
 def test_wgrad_workspace_covers_the_chunk_rule(libpath):
