@@ -194,19 +194,16 @@ int lg_prep_weights(const float* W, int32_t K, int32_t Cin, int32_t Cout, void* 
  * utils/models/minkunet_bev.py:57-123):  Y[out_row[s], :] = out_scale * sum_k A16[nbr[k][s], :] @ B16[wk]^T
  * A16 [n_in][Ck] and B16 [K][N][Ck] are 16-bit (fmt), Ck % 32 == 0, N % 16 == 0, N <= 512.
  * out_scale: nullable device float (undoes lg_absmax_scale).  bias nullable [N].
- * gather_mode: must be 2 = super-tile pipeline (cp.async row gathers arriving on mbarriers, weight panels by TMA,
- *              up to 4 row tiles accumulating in TMEM per weight load; csrc/conv_tc2.cu).  The first-generation
- *              kernels (0 = cp.async, 1 = TMA tile::gather4, measured 2.7x slower) left the library; their source
- *              is kept in tools/legacy/conv_tc_gen1.cu as the record. */
+ * Super-tile pipeline: cp.async row gathers arriving on mbarriers, weight panels by TMA, up to 4 row tiles
+ * accumulating in TMEM per weight load (csrc/conv_tc2.cu). */
 int lg_conv_gemm_tc(const lgConvPlan* plan, const void* A16, int32_t Ck, const void* B16, int32_t N, int32_t flip_k,
-                    int32_t fmt, const float* out_scale, const float* bias, float* Y, int32_t gather_mode,
-                    void* stream);
+                    int32_t fmt, const float* out_scale, const float* bias, float* Y, void* stream);
 
 size_t lg_conv_wgrad_tc_workspace(const lgConvPlan* plan, int32_t Cin, int32_t Cout);
 /* tcgen05 wgrad: dW[k] = out_scale * sum_s X16[nbr[k][s], :]^T dY16[out_row[s], :]  (fp32 [K][Cin][Cout]). */
 int lg_conv_wgrad_tc(const lgConvPlan* plan, const void* X16, int32_t Cin, const void* dY16, int32_t Cout,
-                     int32_t fmt, const float* out_scale, float* dW, int32_t gather_mode, void* workspace,
-                     size_t workspace_bytes, void* stream);
+                     int32_t fmt, const float* out_scale, float* dW, void* workspace, size_t workspace_bytes,
+                     void* stream);
 
 /* ---- layer-level entry points: ONE host call per MinkowskiConvolution each way (same contract as lg_conv_gemm_tc /
  * lg_conv_wgrad_tc; utils/models/minkunet_bev.py:57-123).
@@ -228,11 +225,6 @@ int lg_conv_layer_backward(const lgConvPlan* plan_dgrad, const lgConvPlan* plan_
  * and release (synchronises).  The layer-level calls size it themselves. */
 size_t lg_arena_bytes(void);
 int lg_arena_release(void);
-
-/* Diagnostics of the tensor-core pipeline (tools/prof_roles.py, tools/trace_units.py; active with LIDOG_DBG & 8):
- * per-role wait cycles of CTA 0 (16 counters) and the per-unit event trace [5][512]. */
-int lg_debug_profile(long long* out16, int reset);
-int lg_debug_trace(long long* out);
 
 /* ------------------------------------------------------------------ fused batch norm (+ ReLU, residual, operand cast)
  *

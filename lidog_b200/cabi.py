@@ -74,15 +74,13 @@ SIGNATURES = {
     "lg_cast_rows": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
     "lg_absmax_scale": (C.c_int, [_vp, _i64, _vp, _vp]),
     "lg_prep_weights": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp, _i32, _vp]),
-    "lg_conv_gemm_tc": (C.c_int, [_PP, _vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _vp]),
+    "lg_conv_gemm_tc": (C.c_int, [_PP, _vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp]),
     "lg_conv_wgrad_tc_workspace": (_sz, [_PP, _i32, _i32]),
-    "lg_conv_wgrad_tc": (C.c_int, [_PP, _vp, _i32, _vp, _i32, _i32, _vp, _vp, _i32, _vp, _sz, _vp]),
+    "lg_conv_wgrad_tc": (C.c_int, [_PP, _vp, _i32, _vp, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
     "lg_conv_layer_forward": (C.c_int, [_PP, _vp, _i32, _vp, _i32, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp]),
     "lg_conv_layer_backward": (C.c_int, [_PP, _PP, _i32, _vp, _i32, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _vp]),
     "lg_arena_bytes": (_sz, []),
     "lg_arena_release": (C.c_int, []),
-    "lg_debug_profile": (C.c_int, [_vp, C.c_int]),
-    "lg_debug_trace": (C.c_int, [_vp]),
     "lg_bn_layer_forward": (C.c_int, [_PB, _PB, _vp, _i32, _i64, _i32, _vp, _vp, _i32, _PPC, _vp]),
     "lg_bn_layer_backward": (C.c_int, [_vp, _i64, _vp, _i32, _i64, _i32, _PBB, _PBB, _vp, _i32, _vp, _PPC, _vp]),
     "lg_bn_workspace": (_sz, [_i64, _i32]),

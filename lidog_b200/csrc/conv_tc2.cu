@@ -1,4 +1,4 @@
-// Sparse convolution on tcgen05, second-generation pipeline (gather_mode 2, the default).
+// Sparse convolution on tcgen05: gather-GEMM (forward / dgrad) and wgrad pipelines.
 //
 // Measured on B200 (profiles/r01_conv_bench_v1.txt): tile::gather4 TMA moves 256 B per instruction and
 // sustains ~100 SM cycles per instruction, 2.7x slower than LDGSTS (cp.async) row gathers; and a
@@ -14,7 +14,7 @@
 //     the weight panel W[k] feeds up to T gathered tiles (weight traffic / T);
 //   * wgrad (k_wgrad2): a CTA owns a group of G kernel offsets (G * Cout <= 512 TMEM columns) and a
 //     chunk of tiles; the dY tile is staged once and reused by every offset of the group.
-// Shared-memory operand tiles keep the SWIZZLE_64B layout of conv_tc.cu (64-byte rows = 32 channels).
+// Shared-memory operand tiles use the SWIZZLE_64B layout (64-byte rows = 32 channels).
 // Results are deterministic: every output row / weight element is written once in a fixed order.
 // Reference contract: MinkowskiConvolution(+Transpose) forward/backward, utils/models/minkunet_bev.py:57-123.
 #include <stdlib.h>
@@ -32,22 +32,6 @@ int launch_reduce_partials(const float* partial, int n_chunks, int64_t n_elems, 
 namespace v2 {
 using namespace ptx;
 
-// LIDOG_DBG & 8: CTA 0 accumulates the cycles each role spends waiting (read back by lg_debug_profile)
-__device__ long long g_prof[16];
-// LIDOG_DBG & 8: event trace of CTA 0, [event][unit] = clock64 for the first kTraceUnits units of the launch:
-// 0 producer got the free stage, 1 producer armed the stage barrier, 2 MMA warp saw the stage full, 3 MMA warp
-// committed the unit, 4 id copy issued (read back by lg_debug_trace)
-constexpr int kTraceUnits = 512;
-__device__ long long g_trace[5][kTraceUnits];
-// The instrumentation exists only in the DBG instantiation of the kernel (LIDOG_DBG != 0 selects it): in the
-// production instantiation every macro below compiles to nothing.  (The event trace showed the one-thread MMA role
-// executing ~500 instructions per (offset, panel) step at ~5 cycles each -- it, not the data movement or the tensor
-// pipe, set the pace -- and a third of those instructions were predicated-off instrumentation and switches.)
-#define TRACE(ev, unit) do { if (DBG && prof && (unit) < kTraceUnits) g_trace[ev][unit] = clock64(); } while (0)
-#define PROF_T0() long long _t0 = DBG ? clock64() : 0
-#define PROF_ADD(slot) do { if (DBG && prof) { long long _t1 = clock64(); pacc[slot] += _t1 - _t0; _t0 = _t1; } } while (0)
-#define PROF_FLUSH(lo, hi) do { if (DBG && prof) for (int _i = lo; _i <= hi; ++_i) g_prof[_i] += pacc[_i]; } while (0)
-
 constexpr int kRowB = 64;            // bytes per smem operand row (32 x 16-bit)
 constexpr int kSub = 128 * kRowB;    // one [128 rows x 32 channels] sub-tile = 8 KB
 constexpr int kEpiWarps = 4;         // warps 0..3
@@ -57,12 +41,14 @@ constexpr int kProdWarp0 = 6;
 constexpr int kProdWarps = 4;        // warps 6..9
 constexpr int kIdxWarp = kProdWarp0 + kProdWarps;  // warp 10: row-id ring (bulk copies of 512 B id rows)
 constexpr int kThreads = (kIdxWarp + 1) * 32;
-constexpr int kMma2Warp = kIdxWarp + 1;              // k_gemm2 only: second MMA issuer (SPLIT != 0)
-constexpr int kThreadsG2 = (kMma2Warp + 1) * 32;
 constexpr int kIdxSlotBytes = LG_TILE_ROWS * 4;
+// Row-id ring of k_gemm2.  The ncu source view of the lean kernel (profiles/r01_s4_gemm2_source_stalls.txt) shows the
+// MMA warp polling the stage-full barrier ~17 times per unit and the producers waiting for free stages a quarter of
+// the time -- a latency-bound ring -- so shared memory goes to operand stages first: 16 id slots (8 KB instead of 16).
+constexpr int kGemmIdxSlots = 4 * kProdWarps;
 constexpr int kSchedSlots = 4;                                   // super-tile hand-out ring
 constexpr int kSchedWords = 12;  // ring entry: [0] super-tile, [1] "tile has any offset" bits, [2..9] mask word 0 of its tiles
-constexpr int kSchedConsumers = kEpiWarps + 2 + kProdWarps;      // warps that read every ring entry (+1 with two issuers)
+constexpr int kSchedConsumers = kEpiWarps + 2 + kProdWarps;      // warps that read every ring entry
 constexpr int kStgPitch = 36;                                    // floats per staged row (32 + 4: conflict-free v4)
 constexpr int kStgBytes = kEpiWarps * 32 * kStgPitch * 4;        // epilogue transposition buffers
 
@@ -74,10 +60,6 @@ __device__ __forceinline__ void bulk_copy_g2s(void* dst, const void* src, uint32
                    smem_u32(dst)),
                "l"(src), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
-}
-// L2 prefetch of `bytes` (multiple of 16) at a 16-byte aligned global address: fire and forget
-__device__ __forceinline__ void bulk_prefetch_l2(const void* src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ int lds32(uint32_t saddr) {
   int v;
@@ -209,27 +191,16 @@ struct Gemm2Args {
   const float* out_scale;
   const float* bias;
   int Ck, N, n_blk, flip, umma_fmt;
-  int dbg;  // experiment switches (LIDOG_DBG): 1 = no B loads, 2 = no A copies, 4 = no MMAs, 16 = no proxy fence,
-            // 32 = no result stores, 64 = no row-id copies, 128 = stage release by plain arrive (only with 4);
-            // 8 = per-role cycle counters of CTA 0
   int T, pc, n_panels, sa, sb, np;  // np = active producer warps (<= sa, see the ring-phase note)
-  int ni;                           // row-id ring slots (a multiple of np)
-  int pf;                           // id warp prefetches the operand rows of upcoming units into L2
-  int bmax;                         // units the MMA warp waits for together (one proxy fence per batch), <= sa
-  int sets;                         // accumulator sets in TMEM (sets * T * n_blk <= 512): 2 = the epilogue of one
-                                    // super-tile overlaps the MMAs of the next
   int64_t n_tiles, n_super;
   int* err;
   int* sched;  // [0..3] next super-tile per blockIdx.y, [4] finished CTAs (self-resetting)
 };
 
-// DBG: instrumentation + experiment switches compiled in.  PC: 32-channel chunks per operand stage (= g.pc).
-// SPLIT: MMA issuers.  The one-thread MMA role sets the pace of the kernel (section 4.1 of DESIGN.md), so two
-// warps share it in a way that leaves every accumulator with ONE issuer (deterministic accumulation order):
-//   0 = one issuer; 1 = by tile parity (super-tiles of T >= 2 tiles: warp j issues the units of tiles t = j mod 2);
-//   2 = by column halves (T = 1: both warps issue every unit, warp j the MMAs of columns [j N/2, (j+1) N/2)).
-template <bool DBG, int PC, int SPLIT>
-__global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, const __grid_constant__ CUtensorMap tmB) {
+// PC: 32-channel chunks per operand stage (= g.pc).  TMEM holds two accumulator sets of T tiles (2 * T * n_blk <= 512
+// columns): the epilogue of one super-tile overlaps the MMAs of the next.
+template <int PC>
+__global__ void __launch_bounds__(kThreads, 1) k_gemm2(const Gemm2Args g, const __grid_constant__ CUtensorMap tmB) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -237,7 +208,7 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
   uint8_t* smA = smem;
   uint8_t* smB = smem + (size_t)g.sa * stageA;
   uint8_t* smI = smB + (size_t)g.sb * stageB;  // id ring: ni slots of 128 row ids
-  const int ni = g.ni;
+  constexpr int ni = kGemmIdxSlots;
   float* smStg = (float*)(smI + (size_t)ni * kIdxSlotBytes);  // epilogue transposition buffers
   uint64_t* fullA = (uint64_t*)((uint8_t*)smStg + kStgBytes);
   uint64_t* emptyA = fullA + g.sa;
@@ -254,30 +225,26 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
   SchedCursor sc{0, 0};
   const int n0 = blockIdx.y * g.n_blk;
   const int K = g.plan.kernel_volume;
-  const int dbg = DBG ? g.dbg : 0;  // experiment switches fold away in the production instantiation
-  const bool prof = DBG && (dbg & 8) && blockIdx.x == 0 && blockIdx.y == 0 && lane == 0 && warp != kMma2Warp;
-  long long pacc[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  const long long cta_t0 = DBG ? clock64() : 0;
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < g.sa; ++s) {
       mbar_init(&fullA[s], 32);
-      mbar_init(&emptyA[s], SPLIT == 2 ? 2 : 1);  // column split: both issuers read the stage
+      mbar_init(&emptyA[s], 1);
     }
     for (int s = 0; s < g.sb; ++s) {
       mbar_init(&fullB[s], 1);
-      mbar_init(&emptyB[s], SPLIT ? 2 : 1);  // every issuer releases the weight panel
+      mbar_init(&emptyB[s], 1);
     }
     for (int s = 0; s < ni; ++s) {
       mbar_init(&fullI[s], 1);
       mbar_init(&emptyI[s], 1);
     }
-    mbar_init(&acc_full[0], SPLIT ? 2 : 1);
-    mbar_init(&acc_full[1], SPLIT ? 2 : 1);
+    mbar_init(&acc_full[0], 1);
+    mbar_init(&acc_full[1], 1);
     for (int t = 0; t < 8; ++t) mbar_init(&acc_empty[t], kEpiWarps * 32);
     for (int t = 0; t < kSchedSlots; ++t) {
       mbar_init(&fullS[t], 1);
-      mbar_init(&emptyS[t], kSchedConsumers + (SPLIT ? 1 : 0));
+      mbar_init(&emptyS[t], kSchedConsumers);
     }
     fence_barrier_init();
   }
@@ -292,14 +259,6 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
     // ===================================================================== id ring (runs ahead; one elected lane issues)
     int slot = 0;
     uint32_t iphase = 0;
-    // Optional (LIDOG_G2_OPT & 4, OFF by default): L2 prefetch of the operand rows, kPfLag units behind the id copies
-    // and up to ni - kPfLag units ahead of the gathers.  Measured on B200 (profiles/r01_s4_sweep_b.txt): 128
-    // cp.async.bulk.prefetch.L2 per unit made every layer 1.2-6x SLOWER (0.229 -> 0.834 ms on the block8 shape);
-    // the bulk-prefetch path serialises far below the rate the LDGSTS gathers sustain.  Kept as the record.
-    constexpr int kPfLag = 8;
-    int pslot = 0, pf_count = 0, iunit = 0;
-    uint32_t pphase = 0, pf_hist = 0;
-    const uint32_t row_bytes = (uint32_t)g.Ck * 2u;
     for (;;) {
       mbar_wait(&emptyS[sc.slot], sc.phase ^ 1, g.err, 21);
       int drawn = 0;
@@ -334,41 +293,17 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
         for (int p = 0; p < g.n_panels; ++p) {
           for (uint32_t mm = m; mm; mm &= mm - 1) {
             const int t = __ffs(mm) - 1;
-            if (!(dbg & 512)) mbar_wait(&emptyI[slot], iphase ^ 1, g.err, 7);
-            TRACE(4, iunit);
-            ++iunit;
+            mbar_wait(&emptyI[slot], iphase ^ 1, g.err, 7);
             if (elect_one()) {
-              if (dbg & 64) {  // experiment: no id copies (the producers gather whatever the ring holds)
-                mbar_arrive(&fullI[slot]);
-              } else {
-                mbar_arrive_expect_tx(&fullI[slot], kIdxSlotBytes);
-                bulk_copy_g2s(smI + (size_t)slot * kIdxSlotBytes,
-                              g.plan.nbr + (int64_t)k * g.plan.k_stride + (tile0 + t) * LG_TILE_ROWS, kIdxSlotBytes,
-                              &fullI[slot]);
-              }
+              mbar_arrive_expect_tx(&fullI[slot], kIdxSlotBytes);
+              bulk_copy_g2s(smI + (size_t)slot * kIdxSlotBytes,
+                            g.plan.nbr + (int64_t)k * g.plan.k_stride + (tile0 + t) * LG_TILE_ROWS, kIdxSlotBytes,
+                            &fullI[slot]);
             }
             __syncwarp();
             if (++slot == ni) {
               slot = 0;
               iphase ^= 1;
-            }
-            if (g.pf) {
-              pf_hist = (pf_hist << 1) | (p == 0 ? 1u : 0u);  // later panels of a unit re-read the same rows
-              if (++pf_count > kPfLag) {
-                if ((pf_hist >> kPfLag) & 1u) {
-                  mbar_wait(&fullI[pslot], pphase, g.err, 9);
-                  const int4 ids = *reinterpret_cast<const int4*>(smI + (size_t)pslot * kIdxSlotBytes + lane * 16);
-                  const uint8_t* a = reinterpret_cast<const uint8_t*>(g.A);
-                  if (ids.x >= 0) bulk_prefetch_l2(a + (size_t)ids.x * row_bytes, row_bytes);
-                  if (ids.y >= 0) bulk_prefetch_l2(a + (size_t)ids.y * row_bytes, row_bytes);
-                  if (ids.z >= 0) bulk_prefetch_l2(a + (size_t)ids.z * row_bytes, row_bytes);
-                  if (ids.w >= 0) bulk_prefetch_l2(a + (size_t)ids.w * row_bytes, row_bytes);
-                }
-                if (++pslot == ni) {
-                  pslot = 0;
-                  pphase ^= 1;
-                }
-              }
             }
           }
         }
@@ -377,7 +312,7 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
   } else if (warp >= kProdWarp0 && warp < kProdWarp0 + kProdWarps) {
     // ===================================================================== A producers (cp.async gather)
     const int pw = warp - kProdWarp0;
-    int stage = 0, turn = 0, slot = 0, punit = 0;
+    int stage = 0, turn = 0, slot = 0;
     uint32_t phase = 0, iphase = 0;
     SchedItem item;
     for (;;) {
@@ -392,29 +327,16 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
           for (int t = 0; t < nt; ++t) {
             if (!((m >> t) & 1u)) continue;
             if (turn == pw) {
-              PROF_T0();
               int rows[16];
-              if (!(dbg & 512)) {  // dbg 512: experiment without the id ring on the producer side
-                mbar_wait(&fullI[slot], iphase, g.err, 8);
-                ids_from_ring(rows, smem_u32(smI) + slot * kIdxSlotBytes, lane);
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&emptyI[slot]);
-              }
-              if (pw == 0) PROF_ADD(15);
+              mbar_wait(&fullI[slot], iphase, g.err, 8);
+              ids_from_ring(rows, smem_u32(smI) + slot * kIdxSlotBytes, lane);
+              __syncwarp();
+              if (lane == 0) mbar_arrive(&emptyI[slot]);
               if (lane == 0) mbar_wait(&emptyA[stage], phase ^ 1, g.err, 1);
               __syncwarp();
-              TRACE(0, punit);
-              if (pw == 0) PROF_ADD(0);
-              if (!(dbg & 2))
-                gather_rows<PC>(smA + (size_t)stage * stageA, reinterpret_cast<const uint8_t*>(g.A + p * PC * 32), (uint32_t)g.Ck * 2u, rows, lane);
-              if (dbg & 256)  // experiment (with dbg 2 only): plain arrive instead of the cp.async-tracked one
-                mbar_arrive(&fullA[stage]);
-              else
-                cp_async_arrive_noinc(&fullA[stage]);
-              TRACE(1, punit);
-              if (pw == 0) PROF_ADD(1);
+              gather_rows<PC>(smA + (size_t)stage * stageA, reinterpret_cast<const uint8_t*>(g.A + p * PC * 32), (uint32_t)g.Ck * 2u, rows, lane);
+              cp_async_arrive_noinc(&fullA[stage]);
             }
-            ++punit;
             turn = (turn + 1 == g.np) ? 0 : turn + 1;
             if (++stage == g.sa) {
               stage = 0;
@@ -444,19 +366,13 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
         (void)m;
         const int wk = g.flip ? (K - 1 - k) : k;
         for (int p = 0; p < g.n_panels; ++p) {
-          PROF_T0();
           mbar_wait(&emptyB[bs], bphase ^ 1, g.err, 2);
-          PROF_ADD(2);
           if (elect_one()) {
-            if (dbg & 1) {
-              mbar_arrive(&fullB[bs]);
-            } else {
-              mbar_arrive_expect_tx(&fullB[bs], (uint32_t)stageB);
-              uint8_t* dst = smB + (size_t)bs * stageB;
+            mbar_arrive_expect_tx(&fullB[bs], (uint32_t)stageB);
+            uint8_t* dst = smB + (size_t)bs * stageB;
 #pragma unroll
-              for (int c = 0; c < PC; ++c)
-                tma_load_2d(dst + c * g.n_blk * kRowB, &tmB, (p * PC + c) * 32, wk * g.N + n0, &fullB[bs]);
-            }
+            for (int c = 0; c < PC; ++c)
+              tma_load_2d(dst + c * g.n_blk * kRowB, &tmB, (p * PC + c) * 32, wk * g.N + n0, &fullB[bs]);
           }
           __syncwarp();
           if (++bs == g.sb) {
@@ -466,39 +382,32 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
         }
       }
     }
-  } else if (warp == kMmaWarp || warp == kMma2Warp) {
-    // ===================================================================== MMA issuer(s)
-    const int mw = (warp == kMmaWarp) ? 0 : 1;  // issuer index
-    if (SPLIT == 0 && mw) goto role_done;         // single-issuer instantiation: the extra warp has no role
+  } else if (warp == kMmaWarp) {
+    // ===================================================================== MMA issuer
     // The loop runs warp-uniformly (every lane computes the same unit sequence; the masks are broadcast), and
     // one elected lane issues the tcgen05 instructions: descriptors are a constant high word plus
     // (address >> 4) held in uniform registers, so a unit costs two barrier waits, a proxy fence and 2*pc
     // back-to-back UTCHMMAs.  Accumulators are handed back by the epilogue tile by tile (acc_empty[t]), so
     // the first offsets of the next super-tile overlap the drain of the previous one.
-    // column split: this issuer's MMAs cover n_mma = N/2 columns starting at column col0 (weight rows col0..)
-    const int n_mma = (SPLIT == 2) ? g.n_blk / 2 : g.n_blk;
-    const uint32_t col0 = (SPLIT == 2 && mw) ? (uint32_t)(g.n_blk / 2) : 0u;
-    const uint32_t idesc = make_idesc(g.umma_fmt, 0, 0, LG_TILE_ROWS, n_mma);
+    const uint32_t idesc = make_idesc(g.umma_fmt, 0, 0, LG_TILE_ROWS, g.n_blk);
     const uint64_t desc_hi = make_smem_desc(0, 16, 8 * kRowB, kLayoutSw64);
-    const uint32_t a_base = smem_u32(smA) >> 4, b_base = (smem_u32(smB) + col0 * kRowB) >> 4;
+    const uint32_t a_base = smem_u32(smA) >> 4, b_base = smem_u32(smB) >> 4;
     const uint32_t a_stage16 = (uint32_t)stageA >> 4, b_stage16 = (uint32_t)stageB >> 4;
     const uint32_t b_sub16 = (uint32_t)(g.n_blk * kRowB) >> 4;
     // everything the loop needs lives in registers: no parameter loads, no 64-bit index arithmetic in the hot path
-    const int sa = g.sa, sb = g.sb, T = g.T, n_panels = g.n_panels, n_blk = g.n_blk, two_sets = g.sets == 2;
-    const uint32_t mine_bits = (SPLIT == 1) ? (mw ? 0xAAAAAAAAu : 0x55555555u) : 0xFFFFFFFFu;  // tiles this issuer owns
-    int stage = 0, bs = 0, munit = 0;
+    const int sa = g.sa, sb = g.sb, T = g.T, n_panels = g.n_panels, n_blk = g.n_blk;
+    int stage = 0, bs = 0;
     uint32_t phase = 0, bphase = 0, it = 0;
     SchedItem item;
     for (;;) {
-      PROF_T0();
       sched_next(item, sc, fullS, emptyS, sched_ring, lane, g.err);
       const int64_t st = item.st;
       if (st < 0) break;
       const int64_t tile0 = st * T;
       const int nt = (int)min((int64_t)T, g.n_tiles - tile0);
       if (!item.any) continue;
-      const int set = two_sets ? (int)(it & 1) : 0;
-      const uint32_t eparity = ((two_sets ? (it >> 1) : it) & 1) ^ 1;
+      const int set = (int)(it & 1);
+      const uint32_t eparity = ((it >> 1) & 1) ^ 1;
       const uint32_t d_base = tmem_base + (uint32_t)(set * T) * (uint32_t)n_blk;  // first accumulator of this set
       ++it;
       // all T accumulators of the set are taken up front (the epilogue hands them back tile by tile; the last one
@@ -506,74 +415,45 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
       for (int t = 0; t < T; ++t) mbar_wait(&acc_empty[set * T + t], eparity, g.err, 3);
       uint32_t started = 0;
       TileMasks& tm = item.tm;
-      PROF_ADD(11);
       LG_FOR_EACH_OFFSET(tm, g.plan, tile0, nt, k, m) {
         for (int p = 0; p < n_panels; ++p) {
-          PROF_ADD(7);
           mbar_wait(&fullB[bs], bphase, g.err, 4);
-          PROF_ADD(4);
           const uint32_t db_lo = b_base + bs * b_stage16;
           // The units of this (offset, panel) -- at most T <= ring depth (host-checked) -- are handled together:
           // wait for their stages, ONE proxy fence, issue their MMAs back to back, release the stages.
-          const uint32_t mym = m & mine_bits;  // the units of this step that this issuer handles
           {
             int s = stage;
             uint32_t ph = phase;
             for (uint32_t bb = m; bb; bb &= bb - 1) {
-              // Every issuer observes EVERY phase of every stage barrier, also for the units it does not issue: a
-              // parity wait cannot tell phase n from phase n + 2, and an issuer that skipped the other issuer's
-              // phase and ran >= one ring wrap ahead took the stale completion of its own previous use for the
-              // new one (this is what trapped the tile-parity mode on the 5-stage 96->96 shape).
               mbar_wait(&fullA[s], ph, g.err, 5);
-              TRACE(2, munit + __popc(m & ~bb));
               if (++s == sa) {
                 s = 0;
                 ph ^= 1;
               }
             }
           }
-          PROF_ADD(5);
-          if (!(dbg & 16)) fence_proxy_async();  // cp.async (generic proxy) writes -> tcgen05 (async proxy) reads
+          fence_proxy_async();  // cp.async (generic proxy) writes -> tcgen05 (async proxy) reads
           tc_fence_after();
-          PROF_ADD(10);
           if (elect_one()) {
             int s = stage;
             for (uint32_t bb = m; bb; bb &= bb - 1) {
               const int t = __ffs(bb) - 1;
-              if (SPLIT == 1 && !((mym >> t) & 1u)) {  // the other issuer's unit: only the stage counter moves
-                if (++s == sa) s = 0;
-                continue;
-              }
               const uint64_t da0 = desc_hi | (uint64_t)(a_base + s * a_stage16);
               const uint64_t db0 = desc_hi | (uint64_t)db_lo;
-              const uint32_t d_tmem = d_base + (uint32_t)t * (uint32_t)n_blk + col0;
+              const uint32_t d_tmem = d_base + (uint32_t)t * (uint32_t)n_blk;
               const uint32_t acc0 = (started >> t) & 1u;
-              if (!(dbg & 4)) {
 #pragma unroll
-                for (int c = 0; c < PC; ++c) {
-                  umma_f16(d_tmem, da0 + c * (kSub >> 4), db0 + c * b_sub16, idesc, c == 0 ? acc0 : 1u);
-                  umma_f16(d_tmem, da0 + c * (kSub >> 4) + 2, db0 + c * b_sub16 + 2, idesc, 1u);
-                }
+              for (int c = 0; c < PC; ++c) {
+                umma_f16(d_tmem, da0 + c * (kSub >> 4), db0 + c * b_sub16, idesc, c == 0 ? acc0 : 1u);
+                umma_f16(d_tmem, da0 + c * (kSub >> 4) + 2, db0 + c * b_sub16 + 2, idesc, 1u);
               }
-              if (DBG && (dbg & 128))  // experiment (with dbg 4 only): plain arrive instead of tcgen05.commit
-                mbar_arrive(&emptyA[s]);
-              else
-                umma_commit(&emptyA[s]);
+              umma_commit(&emptyA[s]);
               if (++s == sa) s = 0;
             }
-            if (DBG && (dbg & 128))
-              mbar_arrive(&emptyB[bs]);
-            else
-              umma_commit(&emptyB[bs]);
+            umma_commit(&emptyB[bs]);
           }
           __syncwarp();
-          if (DBG) {
-            for (int i = 0; i < __popc(m); ++i) TRACE(3, munit + i);
-            munit += __popc(m);
-            pacc[13] += __popc(m);  // units
-          }
-          PROF_ADD(6);
-          started |= mym;
+          started |= m;
           stage += __popc(m);
           if (stage >= sa) {
             stage -= sa;
@@ -587,10 +467,7 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
       }
       if (elect_one()) umma_commit(&acc_full[set]);
       __syncwarp();
-      PROF_ADD(3);
-      pacc[14] += 1;  // super-tiles
     }
-    if (DBG) pacc[12] = clock64() - cta_t0;  // lifetime of the MMA role of this CTA
   } else {
     // ===================================================================== epilogue (warps 0..3)
     const float scale = g.out_scale ? g.out_scale[0] : 1.f;
@@ -603,16 +480,14 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
       const int64_t tile0 = st * g.T;
       const int nt = (int)min((int64_t)g.T, g.n_tiles - tile0);
       const uint32_t am = item.any;
-      PROF_T0();
       int a0 = 0;
       if (am) {
-        const int set = (g.sets == 2) ? (int)(it & 1) : 0;
+        const int set = (int)(it & 1);
         a0 = set * g.T;
-        mbar_wait(&acc_full[set], ((g.sets == 2) ? (it >> 1) : it) & 1, g.err, 6);
+        mbar_wait(&acc_full[set], (it >> 1) & 1, g.err, 6);
         ++it;
         tc_fence_after();
       }
-      if (warp == 0) PROF_ADD(8);
       for (int t = 0; t < g.T; ++t) {
         if (t < nt) {
           const int64_t s = (tile0 + t) * LG_TILE_ROWS + warp * 32 + lane;
@@ -679,8 +554,7 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
                   // was measured: the 31 separate adds it removes cost 0.6 ms per step, the loads in this epilogue
                   // 2.8 ms (k_gemm2 8.39 -> 11.17 ms, profiles/r02_c_launch_summary_grad_accum_experiment.txt): the
                   // accumulators drain late and the MMA warp stalls.  Not kept.)
-                  if (!(dbg & 32))  // dbg 32: experiment without the result stores
-                    *reinterpret_cast<float4*>(g.Y + (int64_t)srow[j] * g.N + n0 + n + 4 * (lane & 7)) = o;
+                  *reinterpret_cast<float4*>(g.Y + (int64_t)srow[j] * g.N + n0 + n + 4 * (lane & 7)) = o;
                   cs.x += o.x, cs.y += o.y, cs.z += o.z, cs.w += o.w;
                   cq.x = fmaf(o.x, o.x, cq.x), cq.y = fmaf(o.y, o.y, cq.y), cq.z = fmaf(o.z, o.z, cq.z),
                   cq.w = fmaf(o.w, o.w, cq.w);
@@ -728,16 +602,8 @@ __global__ void __launch_bounds__(kThreadsG2, 1) k_gemm2(const Gemm2Args g, cons
           mbar_arrive(&acc_empty[a0 + t]);
         }
       }
-      if (warp == 0) PROF_ADD(9);
     }
   }
-role_done:
-  if (warp == kProdWarp0) PROF_FLUSH(0, 1);
-  if (warp == kProdWarp0) PROF_FLUSH(15, 15);
-  if (warp == kBWarp) PROF_FLUSH(2, 2);
-  if (warp == kMmaWarp) PROF_FLUSH(3, 7);
-  if (warp == kMmaWarp) PROF_FLUSH(10, 14);  // 11 = schedule hand-out + super-tile prologue of the MMA warp
-  if (warp == 0) PROF_FLUSH(8, 9);
   tc_fence_before();
   __syncthreads();
   if (warp == kMmaWarp) tmem_dealloc(tmem_base, 512);
@@ -762,15 +628,11 @@ struct Wgrad2Args {
   float* partial;  // [chunks][K][Cin][Cout]
   int Cin, Cout, m_blocks, G, n_groups, tiles_per_chunk, umma_fmt, sa, sb, np, bmax;
   int strided;  // offsets of a group are grp + j * n_groups (load balance) instead of a contiguous range
-  int na_max;  // 32-channel sub-blocks per A stage (4; see the launcher for why not min(4, Cin / 32))
-  int dbg;     // DBG instantiation only (LIDOG_WG_DBG): 1 = no dY gathers, 2 = no X gathers, 4 = no MMAs, 8 = no partial stores
   int64_t n_tiles;
   int* err;
 };
 
-template <bool DBG>
 __global__ void __launch_bounds__(kThreads, 1) k_wgrad2(const Wgrad2Args g) {
-  const int dbg = DBG ? g.dbg : 0;  // experiment switches fold away in the production instantiation
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -788,8 +650,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_wgrad2(const Wgrad2Args g) {
   const int na = min(4, (g.Cin - m0) / 32);  // real 32-channel sub-blocks of the A operand
   const int nb = g.Cout / 32;
   // (the MMA always reads 4 sub-blocks = 128 accumulator lanes; lanes of sub-blocks that are not staged hold whatever
-  // the neighbouring stage holds and are never read back: the epilogue stops at Cin)
-  const int stageA = g.na_max * kSub, stageB = nb * kSub;
+  // the stage held before and are never read back: the epilogue stops at Cin)
+  const int stageA = 4 * kSub, stageB = nb * kSub;
   uint8_t* smA = smem;
   uint8_t* smB = smem + (size_t)g.sa * stageA;
   uint8_t* smI = smB + (size_t)g.sb * stageB;  // id ring: ni slots of 128 row ids
@@ -882,7 +744,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wgrad2(const Wgrad2Args g) {
             mbar_wait(&emptyA[stage], phase ^ 1, g.err, 11);
           }
           __syncwarp();
-          if (!(dbg & 2)) gather_stage(smA + (size_t)stage * stageA, g.X, g.Cin, m0, na, rows, lane);
+          gather_stage(smA + (size_t)stage * stageA, g.X, g.Cin, m0, na, rows, lane);
           cp_async_arrive_noinc(&fullA[stage]);
         }
         turn = (turn + 1 == g.np) ? 0 : turn + 1;
@@ -925,9 +787,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_wgrad2(const Wgrad2Args g) {
       if (lane == 0) mbar_wait(&emptyB[bs], bphase ^ 1, g.err, 12);
       __syncwarp();
       uint8_t* dst = smB + (size_t)bs * stageB;
-      if (!(dbg & 1))
-        for (int c0 = 0; c0 < nb; c0 += 4)
-          gather_stage(dst + c0 * kSub, g.dY, g.Cout, c0 * 32, min(4, nb - c0), rows, lane);
+      for (int c0 = 0; c0 < nb; c0 += 4)
+        gather_stage(dst + c0 * kSub, g.dY, g.Cout, c0 * 32, min(4, nb - c0), rows, lane);
       cp_async_arrive_noinc(&fullB[bs]);
       if (++bs == g.sb) {
         bs = 0;
@@ -983,12 +844,10 @@ __global__ void __launch_bounds__(kThreads, 1) k_wgrad2(const Wgrad2Args g) {
             const uint64_t da0 = desc_hi | (uint64_t)(a_base + s * a_stage16);
             const uint32_t d_tmem = tmem_base + j * g.Cout;
             const uint32_t acc0 = (started >> j) & 1u;
-            if (!(dbg & 4)) {
-              umma_f16(d_tmem, da0, db0, idesc, acc0);
+            umma_f16(d_tmem, da0, db0, idesc, acc0);
 #pragma unroll
-              for (int q = 1; q < LG_TILE_ROWS / 16; ++q)  // K = 16 gathered rows per MMA
-                umma_f16(d_tmem, da0 + q * (16 * kRowB >> 4), db0 + q * (16 * kRowB >> 4), idesc, 1u);
-            }
+            for (int q = 1; q < LG_TILE_ROWS / 16; ++q)  // K = 16 gathered rows per MMA
+              umma_f16(d_tmem, da0 + q * (16 * kRowB >> 4), db0 + q * (16 * kRowB >> 4), idesc, 1u);
             umma_commit(&emptyA[s]);
             if (++s == g.sa) s = 0;
           }
@@ -1037,7 +896,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_wgrad2(const Wgrad2Args g) {
 #pragma unroll
           for (int q = 0; q < 16; ++q) v[q] = 0u;
         }
-        if (ci < g.Cin && !(dbg & 8)) {
+        if (ci < g.Cin) {
 #pragma unroll
           for (int q = 0; q < 4; ++q)
             *reinterpret_cast<float4*>(prow + n + 4 * q) =
@@ -1058,52 +917,96 @@ static inline size_t wgrad_tail_bytes(int sa, int sb) {  // id ring + barriers +
   const int ni = 8 * kProdWarps;
   return (size_t)ni * kIdxSlotBytes + (size_t)(2 * sa + 2 * sb + 2 * ni + 2) * 8 + 16 + 1024;
 }
-static inline size_t tail_bytes(int sa, int sb, int ni = 8 * kProdWarps) {  // + epilogue staging + schedule ring
+static inline size_t tail_bytes(int sa, int sb) {  // + epilogue staging + schedule ring
+  const int ni = kGemmIdxSlots;
   return (size_t)ni * kIdxSlotBytes + kStgBytes + (size_t)(2 * sa + 2 * sb + 2 * ni + 11 + 2 * kSchedSlots) * 8 + 16 +
          4 * kSchedWords * kSchedSlots + 1024;
 }
 
-}  // namespace v2
+// Launch shape of k_gemm2, a pure function of the problem: grid (min(n_super, sm_count), n_split) x kThreads, smem bytes.
+struct Gemm2Shape {
+  int n_split, n_blk;  // column blocks of N (blockIdx.y) and their width
+  int T, pc, n_panels, sa, sb, np;  // see Gemm2Args
+  int64_t n_super;
+  size_t smem;
+};
 
-int debug_profile(long long* out16, int reset) {
-  if (out16) LG_CUDA_OK(cudaMemcpyFromSymbol(out16, v2::g_prof, sizeof(long long) * 16));
-  if (reset) {
-    long long z[16] = {0};
-    LG_CUDA_OK(cudaMemcpyToSymbol(v2::g_prof, z, sizeof(z)));
+static int gemm2_shape(int64_t n_tiles, int Ck, int N, int sm_count, bool stats, Gemm2Shape* s) {
+  s->n_split = (N + 255) / 256;
+  s->n_blk = N / s->n_split;
+  if (s->n_blk % 16 != 0 || s->n_blk * s->n_split != N) {
+    set_error("lg_conv_gemm_tc: N=%d cannot be split into equal multiples of 16", N);
+    return LG_ERR_UNSUPPORTED;
+  }
+  if (stats && s->n_blk % 32 != 0) {
+    set_error("lg_conv_layer_forward: epilogue statistics need column blocks that are multiples of 32 (N=%d)", N);
+    return LG_ERR_UNSUPPORTED;
+  }
+  if (s->n_split > 4) {
+    set_error("lg_conv_gemm_tc: N=%d needs more than 4 column blocks", N);
+    return LG_ERR_UNSUPPORTED;
+  }
+  const int n_chunks = Ck / 32;
+  s->n_panels = (n_chunks + 3) / 4;
+  while (n_chunks % s->n_panels != 0) ++s->n_panels;
+  s->pc = n_chunks / s->n_panels;
+  // Tiles per super-tile.  TMEM holds two accumulator sets of T tiles, 2 * T * n_blk <= 512 columns (n_blk <= 256 by
+  // the split above, so T >= 1 always fits), and 2 * T <= 8 accumulator barriers; but keep >= ~3 super-tiles per SM.
+  int T = 256 / s->n_blk < 4 ? 256 / s->n_blk : 4;
+  while (T > 1 && ceil_div(n_tiles, T) * s->n_split < 3 * (int64_t)sm_count) --T;
+  // Pipeline shape.  The weight-panel ring gets 3 stages whenever 4 operand stages still fit next to it (with 2,
+  // the TMA load of the next panel cannot start before the MMAs of the current one retire: the 256-channel
+  // layers waited 22 % of the time for weights); the rest of the budget goes to operand (gather) stages.
+  size_t stageA, stageB;
+  for (;;) {
+    stageA = (size_t)s->pc * kSub, stageB = (size_t)s->pc * s->n_blk * kRowB;
+    s->sb = (3 * stageB + 4 * stageA + tail_bytes(4, 3) <= kSmemBudget) ? 3 : 2;
+    s->sa = 12;
+    while (s->sa > 2 && s->sa * stageA + s->sb * stageB + tail_bytes(s->sa, s->sb) > kSmemBudget) --s->sa;
+    // would 2 weight stages buy an operand stage?  Only where a weight stage is no bigger than an operand stage:
+    // measured (profiles/r01_s4_sweep_n_ring.txt) -17 % / -12 % on the 128-channel layers at tensor stride 8 / 4,
+    // but +2 ... +5 % on the 256-channel single-tile layers, whose 32 KB panels want the third stage.
+    if (s->sb == 3 && s->sa < 12 && stageB <= stageA) {
+      int sa2 = 12;
+      while (sa2 > 2 && sa2 * stageA + 2 * stageB + tail_bytes(sa2, 2) > kSmemBudget) --sa2;
+      if (sa2 > s->sa) {
+        s->sa = sa2;
+        s->sb = 2;
+      }
+    }
+    if (s->sa >= kProdWarps || s->pc == 1) break;
+    // deeper ring with smaller panels (pc must divide the chunk count)
+    int pc = s->pc - 1;
+    while (n_chunks % pc != 0) --pc;
+    s->pc = pc;
+    s->n_panels = n_chunks / pc;
+  }
+  s->T = T < s->sa ? T : s->sa;  // the MMA warp waits for up to T stages at once: they must all fit in the ring
+  s->n_super = ceil_div(n_tiles, s->T);
+  // Ring-phase rule: a producer warp revisits a stage only after the consumer freed it once, which the
+  // parity wait can tell only when consecutive units of one warp are < one ring wrap apart: np <= sa.
+  s->np = s->sa < kProdWarps ? s->sa : kProdWarps;
+  s->smem = s->sa * stageA + s->sb * stageB + tail_bytes(s->sa, s->sb);
+  if (s->smem > kSmemBudget) {
+    set_error("lg_conv_gemm_tc: shared memory %zu exceeds the budget (Ck=%d N=%d)", s->smem, Ck, N);
+    return LG_ERR_UNSUPPORTED;
   }
   return LG_OK;
 }
 
-// Experiment switches, read ONCE per process (they used to cost ~10 getenv calls per launch):
-//   LIDOG_DBG        instrumented instantiation + experiment bits (see Gemm2Args::dbg)
-//   LIDOG_ACC_SETS   1 = single accumulator set
-//   LIDOG_G2_OPT     bit 2 = deep weight-panel ring, bit 4 = L2 row prefetch (measured slower, off)
-//   LIDOG_G2_SB / LIDOG_G2_PC   pin the panel-ring depth / 32-channel chunks per operand stage
-//   LIDOG_G2_RING    0 = the ring shape of the first validated lean kernel (32 id slots, 3 weight stages when they fit)
-//   LIDOG_G2_T       pin the tiles per super-tile (parity tests sweep the multi-tile schedules on small inputs)
-//   LIDOG_WG_CTAS / LIDOG_WG_BATCH / LIDOG_WG_SB   wgrad CTA target / MMA-warp batch / dY ring depth
-//   LIDOG_WG_STRIDED 0 = contiguous offset groups (round 1)
-struct Switches {
-  int dbg, acc_sets, opt, force_sb, force_pc, ring_new, force_t, wg_ctas, wg_batch, mma2, wg_sb, wg_na4, wg_sa, wg_dbg, wg_strided;
-};
-static const Switches& switches() {
-  static const Switches sw = {env_int("LIDOG_DBG", 0),     env_int("LIDOG_ACC_SETS", 2), env_int("LIDOG_G2_OPT", 3),
-                              env_int("LIDOG_G2_SB", 0),   env_int("LIDOG_G2_PC", 0),    env_int("LIDOG_G2_RING", 1) != 0,
-                              env_int("LIDOG_G2_T", 0),    env_int("LIDOG_WG_CTAS", 0),  env_int("LIDOG_WG_BATCH", 4),
-                              env_int("LIDOG_G2_MMA2", 0), env_int("LIDOG_WG_SB", 0),
-                              env_int("LIDOG_WG_NA4", 1),  env_int("LIDOG_WG_SA", 0),
-                              env_int("LIDOG_WG_DBG", 0),  env_int("LIDOG_WG_STRIDED", 1)};
-  return sw;
-}
+}  // namespace v2
 
 // host launcher: forward / dgrad
 int launch_gemm_tc2(const lgConvPlan* plan, const void* A16, int Ck, const void* B16, int N, int flip_k, int fmt,
                     const float* out_scale, const float* bias, float* Y, float* stats, cudaStream_t stream) {
   using namespace v2;
-  const Switches& sw = switches();
   int sm_count = 0;
   int* err = nullptr;
   int rc = tc_runtime(&sm_count, &err);
+  if (rc) return rc;
+  const int64_t n_tiles = plan->n_slots / LG_TILE_ROWS;
+  Gemm2Shape s;
+  rc = gemm2_shape(n_tiles, Ck, N, sm_count, stats != nullptr, &s);
   if (rc) return rc;
   Gemm2Args g;
   g.plan = *plan;
@@ -1114,149 +1017,37 @@ int launch_gemm_tc2(const lgConvPlan* plan, const void* A16, int Ck, const void*
   g.bias = bias;
   g.Ck = Ck;
   g.N = N;
-  const int n_split = (N + 255) / 256;
-  g.n_blk = N / n_split;
-  if (g.n_blk % 16 != 0 || g.n_blk * n_split != N) {
-    set_error("lg_conv_gemm_tc: N=%d cannot be split into equal multiples of 16", N);
-    return LG_ERR_UNSUPPORTED;
-  }
-  if (stats && g.n_blk % 32 != 0) {
-    set_error("lg_conv_layer_forward: epilogue statistics need column blocks that are multiples of 32 (N=%d)", N);
-    return LG_ERR_UNSUPPORTED;
-  }
+  g.n_blk = s.n_blk;
   g.flip = flip_k;
-  g.dbg = sw.dbg;
   g.umma_fmt = (fmt == LG_FMT_BF16) ? 1 : 0;
-  g.n_tiles = plan->n_slots / LG_TILE_ROWS;
+  g.T = s.T;
+  g.pc = s.pc;
+  g.n_panels = s.n_panels;
+  g.sa = s.sa;
+  g.sb = s.sb;
+  g.np = s.np;
+  g.n_tiles = n_tiles;
+  g.n_super = s.n_super;
   g.err = err;
   rc = counter_slot(&g.sched);
   if (rc) return rc;
-  if (n_split > 4) {
-    set_error("lg_conv_gemm_tc: N=%d needs more than 4 column blocks", N);
-    return LG_ERR_UNSUPPORTED;
-  }
-  const int n_chunks = Ck / 32;
-  g.n_panels = (n_chunks + 3) / 4;
-  while (n_chunks % g.n_panels != 0) ++g.n_panels;
-  g.pc = n_chunks / g.n_panels;
-  // tiles per super-tile: as many accumulators as TMEM holds (<= 8), but keep >= ~3 super-tiles per SM
-  int T = 512 / g.n_blk;
-  if (T > 8) T = 8;
-  while (T > 1 && ceil_div(g.n_tiles, T) * n_split < 3 * (int64_t)sm_count) --T;
-  if (sw.force_t > 0 && sw.force_t < T) T = sw.force_t;
-  if (sw.force_t > T && sw.force_t <= 8 && sw.force_t * g.n_blk <= 512) T = sw.force_t;
-  // two accumulator sets when that still leaves T >= 1 (LIDOG_ACC_SETS=1 forces the single-set schedule)
-  g.sets = 1;
-  if (sw.acc_sets == 2 && 2 * g.n_blk <= 512) {
-    g.sets = 2;
-    const int tmax = 512 / (2 * g.n_blk) < 4 ? 512 / (2 * g.n_blk) : 4;  // 2 * T accumulator barriers <= 8
-    if (T > tmax) T = tmax;
-  }
-  g.T = T;
-  g.n_super = ceil_div(g.n_tiles, T);
-  // Pipeline shape.  The weight-panel ring gets 3 stages whenever 4 operand stages still fit next to it (with 2,
-  // the TMA load of the next panel cannot start before the MMAs of the current one retire: the 256-channel
-  // layers waited 22 % of the time for weights); the rest of the budget goes to operand (gather) stages.
-  const int opt = sw.opt;
-  const int force_sb = sw.force_sb, force_pc = sw.force_pc;
-  if (force_pc > 0 && force_pc < g.pc) {
-    int pc = force_pc;
-    while (n_chunks % pc != 0) --pc;
-    g.pc = pc;
-    g.n_panels = n_chunks / pc;
-  }
-  // Ring shape (LIDOG_G2_RING=0 restores 32 id slots / 3 weight stages).  The ncu source view of the lean kernel
-  // (profiles/r01_s4_gemm2_source_stalls.txt) shows the MMA warp polling the stage-full barrier ~17 times per unit
-  // and the producers waiting for free stages a quarter of the time -- a latency-bound ring -- so shared memory goes
-  // to operand stages first: 16 id slots (8 KB instead of 16) and 2 weight stages whenever that buys another stage.
-  const int ring_new = sw.ring_new;
-  const int ni_slots = ring_new ? 4 * kProdWarps : 8 * kProdWarps;
-  size_t stageA, stageB;
-  for (;;) {
-    stageA = (size_t)g.pc * kSub, stageB = (size_t)g.pc * g.n_blk * kRowB;
-    if (force_sb >= 2)
-      g.sb = force_sb;
-    else if (opt & 2)
-      g.sb = (3 * stageB + 4 * stageA + tail_bytes(4, 3, ni_slots) <= kSmemBudget) ? 3 : 2;
-    else
-      g.sb = (3 * stageB <= 80 * 1024) ? 3 : 2;
-    g.sa = 12;
-    while (g.sa > 2 && g.sa * stageA + g.sb * stageB + tail_bytes(g.sa, g.sb, ni_slots) > kSmemBudget) --g.sa;
-    // would 2 weight stages buy an operand stage?  Only where a weight stage is no bigger than an operand stage:
-    // measured (profiles/r01_s4_sweep_n_ring.txt) -17 % / -12 % on the 128-channel layers at tensor stride 8 / 4,
-    // but +2 ... +5 % on the 256-channel single-tile layers, whose 32 KB panels want the third stage.
-    if (ring_new && force_sb < 2 && g.sb == 3 && g.sa < 12 && stageB <= stageA) {
-      int sa2 = 12;
-      while (sa2 > 2 && sa2 * stageA + 2 * stageB + tail_bytes(sa2, 2, ni_slots) > kSmemBudget) --sa2;
-      if (sa2 > g.sa) {
-        g.sa = sa2;
-        g.sb = 2;
-      }
-    }
-    if (g.sa >= kProdWarps || g.pc == 1) break;
-    // deeper ring with smaller panels (pc must divide the chunk count)
-    int pc = g.pc - 1;
-    while (n_chunks % pc != 0) --pc;
-    g.pc = pc;
-    g.n_panels = n_chunks / pc;
-  }
-  g.bmax = 0;  // (unused since the MMA warp takes all units of an (offset, panel) step together)
-  g.pf = (opt & 4) ? 1 : 0;
-  if (g.T > g.sa) {  // the MMA warp waits for up to T stages at once: they must all fit in the ring
-    g.T = g.sa;
-    g.n_super = ceil_div(g.n_tiles, g.T);
-  }
-  // Ring-phase rule: a producer warp revisits a stage only after the consumer freed it once, which the
-  // parity wait can tell only when consecutive units of one warp are < one ring wrap apart: np <= sa.
-  g.np = g.sa < kProdWarps ? g.sa : kProdWarps;
-  g.ni = ni_slots;
-  const size_t smem = g.sa * stageA + g.sb * stageB + tail_bytes(g.sa, g.sb, ni_slots);
-  if (smem > kSmemBudget) {
-    set_error("lg_conv_gemm_tc: shared memory %zu exceeds the budget (Ck=%d N=%d)", smem, Ck, N);
-    return LG_ERR_UNSUPPORTED;
-  }
   CUtensorMap tmB;
   memset(&tmB, 0, sizeof(tmB));
   rc = tc_make_tmap(&tmB, B16, (int64_t)plan->kernel_volume * N, Ck, g.n_blk);
   if (rc) return rc;
-  dim3 grid((unsigned)(g.n_super < sm_count ? g.n_super : sm_count), (unsigned)n_split);
-  // One production instantiation per stage width.  The two-issuer modes (SPLIT 1 / 2) are EXPERIMENTAL and compiled
-  // only with -DLIDOG_EXPERIMENTAL (then LIDOG_G2_MMA2=1 selects them): measured <= 6 % where they ran, and the
-  // tile-parity mode trapped on one shape before the every-phase wait fix, which is unverified on hardware.
-  int split = 0;
-#ifdef LIDOG_EXPERIMENTAL
-  if (sw.mma2) split = g.T >= 2 ? 1 : ((g.n_blk % 32 == 0) ? 2 : 0);
-#endif
-#define LG_LAUNCH_GEMM2(DBGV, PCV, SPV)                                                                                   \
-  do {                                                                                                                     \
-    LG_CUDA_OK(cudaFuncSetAttribute(k_gemm2<DBGV, PCV, SPV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));    \
-    k_gemm2<DBGV, PCV, SPV><<<grid, kThreadsG2, smem, stream>>>(g, tmB);                                                   \
+  const dim3 grid((unsigned)(s.n_super < sm_count ? s.n_super : sm_count), (unsigned)s.n_split);
+  const size_t smem = s.smem;
+#define LG_LAUNCH_GEMM2(PCV)                                                                                   \
+  do {                                                                                                         \
+    LG_CUDA_OK(cudaFuncSetAttribute(k_gemm2<PCV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
+    k_gemm2<PCV><<<grid, kThreads, smem, stream>>>(g, tmB);                                                    \
   } while (0)
-#ifdef LIDOG_EXPERIMENTAL
-#define LG_LAUNCH_GEMM2_SP(DBGV, PCV)                                                                                      \
-  switch (split) {                                                                                                         \
-    case 0: LG_LAUNCH_GEMM2(DBGV, PCV, 0); break;                                                                          \
-    case 1: LG_LAUNCH_GEMM2(DBGV, PCV, 1); break;                                                                          \
-    default: LG_LAUNCH_GEMM2(DBGV, PCV, 2); break;                                                                         \
+  switch (g.pc) {
+    case 1: LG_LAUNCH_GEMM2(1); break;
+    case 2: LG_LAUNCH_GEMM2(2); break;
+    case 3: LG_LAUNCH_GEMM2(3); break;
+    default: LG_LAUNCH_GEMM2(4); break;
   }
-#else
-#define LG_LAUNCH_GEMM2_SP(DBGV, PCV) LG_LAUNCH_GEMM2(DBGV, PCV, 0);
-#endif
-#define LG_LAUNCH_GEMM2_PC(DBGV)                                                                                           \
-  switch (g.pc) {                                                                                                          \
-    case 1: LG_LAUNCH_GEMM2_SP(DBGV, 1); break;                                                                            \
-    case 2: LG_LAUNCH_GEMM2_SP(DBGV, 2); break;                                                                            \
-    case 3: LG_LAUNCH_GEMM2_SP(DBGV, 3); break;                                                                            \
-    default: LG_LAUNCH_GEMM2_SP(DBGV, 4); break;                                                                           \
-  }
-  (void)split;
-  if (g.dbg) {
-    LG_LAUNCH_GEMM2_PC(true)
-  } else {
-    LG_LAUNCH_GEMM2_PC(false)
-  }
-#undef LG_LAUNCH_GEMM2_PC
-#undef LG_LAUNCH_GEMM2_SP
 #undef LG_LAUNCH_GEMM2
   LG_LAUNCH_OK();
   return LG_OK;
@@ -1275,17 +1066,11 @@ static int wgrad2_shape(const lgConvPlan* plan, int Cin, int Cout, int* G, int* 
   // re-read by the reduction) and one pipeline ramp, so a chunk should own >= ~32 tiles; but the launch wants at
   // least one wave of 148 CTAs and gains nothing beyond four.  Measured (profiles/r01_s4_sweep_a.txt): the layers at
   // tensor stride >= 4 ran 1.3-1.8x faster with 148 CTAs than with 592, the stride-1 layers 1.3x slower.
-  const int target_ctas = switches().wg_ctas;
   const int64_t per = (int64_t)*n_groups * m_blocks;
-  int64_t want;
-  if (target_ctas > 0) {
-    want = target_ctas / per;
-  } else {
-    const int64_t hi = 592 / per, lo = ceil_div((int64_t)148, per);
-    want = n_tiles / 32;
-    if (want < lo) want = lo;
-    if (want > hi) want = hi;
-  }
+  const int64_t hi = 592 / per, lo = ceil_div((int64_t)148, per);
+  int64_t want = n_tiles / 32;
+  if (want < lo) want = lo;
+  if (want > hi) want = hi;
   if (want < 1) want = 1;
   int64_t chunks = n_tiles < want ? n_tiles : want;
   if (chunks < 1) chunks = 1;
@@ -1318,44 +1103,33 @@ int launch_wgrad_tc2(const lgConvPlan* plan, const void* X16, int Cin, const voi
   g.umma_fmt = (fmt == LG_FMT_BF16) ? 1 : 0;
   g.n_tiles = plan->n_slots / LG_TILE_ROWS;
   g.err = err;
-  // An X stage always holds 4 sub-blocks (32 KB) although a 96-channel layer fills 3 and a 32-channel layer 1.
-  // Packing the stages tighter (LIDOG_WG_NA4=0) is WRONG: the M = 128 MMA then reads its unused sub-blocks out of
-  // the neighbouring stages, and the full-scale parity test (tests/test_gpu_fullscale.py) measured 0.3-2.5 % error in
-  // dW -- bisected on hardware (profiles/r02_b_wgrad_bisect.log); the switch stays for that record only.
-  g.na_max = switches().wg_na4 ? 4 : (Cin / 32 < 4 ? Cin / 32 : 4);
   // strided groups where there are enough groups for the imbalance to matter: measured -7 ... -20 % on the 96- / 128- /
   // 256-channel layers (5 ... 14 groups), +15 % on the 32-channel ones (4 groups of 7 offsets, already balanced, and
   // every extra dY tile load is pure HBM cost there) -- profiles/r02_d_layer_table_strided.txt
-  g.strided = (switches().wg_strided && g.n_groups >= 5) ? 1 : 0;
+  g.strided = g.n_groups >= 5 ? 1 : 0;
   if (plan->kernel_volume > 64) {
     set_error("lg_conv_wgrad_tc: kernel volume %d > 64 is not on the tensor-core path", plan->kernel_volume);
     return LG_ERR_UNSUPPORTED;
   }
-  const size_t stageA = (size_t)g.na_max * kSub, stageB = (size_t)(Cout / 32) * kSub;
+  // An X stage always holds 4 sub-blocks (32 KB) although a 96-channel layer fills 3 and a 32-channel layer 1.
+  // Packing the stages tighter is WRONG: the M = 128 MMA then reads its unused sub-blocks out of the neighbouring
+  // stages, and the full-scale parity test (tests/test_gpu_fullscale.py) measured 0.3-2.5 % error in dW -- bisected
+  // on hardware (profiles/r02_b_wgrad_bisect.log).
+  const size_t stageA = 4 * kSub, stageB = (size_t)(Cout / 32) * kSub;
   // dY ring: 3 stages when 4 X stages still fit next to them (the MMA warp waited on this ring, see the dY producer)
   g.sb = (4 * stageA + 3 * stageB + wgrad_tail_bytes(4, 3) <= kSmemBudget) ? 3 : 2;
-  if (switches().wg_sb >= 2) g.sb = switches().wg_sb;
-  g.sa = switches().wg_sa >= 2 ? switches().wg_sa : 6;
+  g.sa = 6;
   while (g.sa > 2 && g.sa * stageA + g.sb * stageB + wgrad_tail_bytes(g.sa, g.sb) > kSmemBudget) --g.sa;
   g.np = g.sa < kProdWarps ? g.sa : kProdWarps;
-  {
-    const int want = switches().wg_batch;
-    g.bmax = want < 1 ? 1 : (want < g.sa ? want : g.sa);
-  }
+  g.bmax = g.sa < 4 ? g.sa : 4;  // offsets of a tile per batch of the MMA warp
   const size_t smem = g.sa * stageA + g.sb * stageB + wgrad_tail_bytes(g.sa, g.sb);
   if (smem > kSmemBudget) {
     set_error("lg_conv_wgrad_tc: shared memory %zu exceeds the budget (Cin=%d Cout=%d)", smem, Cin, Cout);
     return LG_ERR_UNSUPPORTED;
   }
   dim3 grid((unsigned)(g.n_groups * g.m_blocks), (unsigned)chunks);
-  g.dbg = switches().wg_dbg;
-  if (g.dbg) {
-    LG_CUDA_OK(cudaFuncSetAttribute(k_wgrad2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_wgrad2<true><<<grid, kThreads, smem, stream>>>(g);
-  } else {
-    LG_CUDA_OK(cudaFuncSetAttribute(k_wgrad2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_wgrad2<false><<<grid, kThreads, smem, stream>>>(g);
-  }
+  LG_CUDA_OK(cudaFuncSetAttribute(k_wgrad2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_wgrad2<<<grid, kThreads, smem, stream>>>(g);
   LG_LAUNCH_OK();
   return launch_reduce_partials((const float*)workspace, chunks, (int64_t)plan->kernel_volume * Cin * Cout, out_scale,
                                 dW, stream);
@@ -1411,15 +1185,10 @@ using namespace lg;
 
 extern "C" int lg_conv_gemm_tc(const lgConvPlan* plan, const void* A16, int32_t Ck, const void* B16, int32_t N,
                                int32_t flip_k, int32_t fmt, const float* out_scale, const float* bias, float* Y,
-                               int32_t gather_mode, void* stream_) {
+                               void* stream_) {
   int rc = check_gemm(plan, Ck, N, fmt, "lg_conv_gemm_tc");
   if (rc) return rc;
   LG_CHECK_ARG(A16 && B16 && Y, "lg_conv_gemm_tc: null pointer");
-  if (gather_mode != 2) {
-    set_error("lg_conv_gemm_tc: gather_mode %d is not in the library (the first-generation kernels live in "
-              "tools/legacy/conv_tc_gen1.cu as the record)", gather_mode);
-    return LG_ERR_UNSUPPORTED;
-  }
   return launch_gemm_tc2(plan, A16, Ck, B16, N, flip_k, fmt, out_scale, bias, Y, nullptr, (cudaStream_t)stream_);
 }
 
@@ -1429,16 +1198,12 @@ extern "C" size_t lg_conv_wgrad_tc_workspace(const lgConvPlan* plan, int32_t Cin
 }
 
 extern "C" int lg_conv_wgrad_tc(const lgConvPlan* plan, const void* X16, int32_t Cin, const void* dY16, int32_t Cout,
-                                int32_t fmt, const float* out_scale, float* dW, int32_t gather_mode, void* workspace,
-                                size_t workspace_bytes, void* stream_) {
+                                int32_t fmt, const float* out_scale, float* dW, void* workspace, size_t workspace_bytes,
+                                void* stream_) {
   int rc = check_wgrad(plan, Cin, Cout, fmt, "lg_conv_wgrad_tc");
   if (rc) return rc;
   LG_CHECK_ARG(X16 && dY16 && dW && workspace, "lg_conv_wgrad_tc: null pointer");
   LG_CHECK_ARG(workspace_bytes >= lg_conv_wgrad_tc_workspace(plan, Cin, Cout), "lg_conv_wgrad_tc: workspace too small");
-  if (gather_mode != 2) {
-    set_error("lg_conv_wgrad_tc: gather_mode %d is not in the library", gather_mode);
-    return LG_ERR_UNSUPPORTED;
-  }
   return launch_wgrad_tc2(plan, X16, Cin, dY16, Cout, fmt, out_scale, dW, workspace, (cudaStream_t)stream_);
 }
 
@@ -1481,13 +1246,5 @@ extern "C" int lg_conv_layer_backward(const lgConvPlan* plan_dgrad, const lgConv
     rc = launch_wgrad_tc2(plan_wgrad, X16, Cin, dY16, Cout, fmt, inv_scale, dW, arena_take(&ar, ws), stream);
     if (rc) return rc;
   }
-  return LG_OK;
-}
-
-// experiment hook (not part of the reference-facing ABI): per-role wait cycles of CTA 0, LIDOG_DBG & 8
-extern "C" int lg_debug_profile(long long* out16, int reset) { return lg::debug_profile(out16, reset); }
-// event trace of CTA 0 (LIDOG_DBG & 8): out[5][512] clock64 values, see g_trace
-extern "C" int lg_debug_trace(long long* out) {
-  if (cudaMemcpyFromSymbol(out, lg::v2::g_trace, sizeof(long long) * 5 * lg::v2::kTraceUnits) != cudaSuccess) return LG_ERR_CUDA;
   return LG_OK;
 }

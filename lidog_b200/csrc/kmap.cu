@@ -7,7 +7,6 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include "common.cuh"
-#include "runtime.cuh"
 #include "scan.cuh"
 
 namespace lg {
@@ -131,8 +130,7 @@ __global__ void __launch_bounds__(LG_TILE_ROWS)
 }
 
 static bool neighbors_symmetric(int same_set, int kernel_size) {
-  static const int sym_on = env_int("LIDOG_KMAP_SYM", 1);
-  return same_set && sym_on && (kernel_size & 1) && kernel_size >= 3;
+  return same_set && (kernel_size & 1) && kernel_size >= 3;
 }
 
 static int launch_neighbors(const void* table_in, int64_t capacity_in, const int32_t* out_coords4, int64_t n_out,

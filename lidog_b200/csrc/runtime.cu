@@ -46,10 +46,6 @@ int device_rt(DeviceRt** out) {
   DeviceRt& r = g_rt[dev];
   if (!r.ready) {
     LG_CUDA_OK(cudaDeviceGetAttribute(&r.sm_count, cudaDevAttrMultiProcessorCount, dev));
-    // Experiment switch: persistent grids leave this many SMs free (for NCCL's CTAs under DDP; a persistent CTA queued
-    // behind a long all-reduce CTA delays the completion of its whole grid).
-    int reserve = env_int("LIDOG_SM_RESERVE", 0);
-    if (reserve > 0 && reserve < r.sm_count) r.sm_count -= reserve;
     LG_CUDA_OK(cudaMalloc(&r.err_word, sizeof(int)));
     LG_CUDA_OK(cudaMemset(r.err_word, 0, sizeof(int)));
     LG_CUDA_OK(cudaMalloc(&r.counters, kCounterSlots * 8 * sizeof(int)));
@@ -182,12 +178,6 @@ int tc_make_tmap(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, i
     return LG_ERR_CUDA;
   }
   return LG_OK;
-}
-
-// Environment switches are read once per process (they select experiments, not behaviour the caller controls).
-int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
 }
 
 }  // namespace lg

@@ -11,7 +11,6 @@ namespace lg {
 int tc_runtime(int* sm_count, int** err_word);
 int counter_slot(int** out);  // 8 zeroed ints the kernel must leave zeroed (schedule counters, last-block tickets)
 int tc_make_tmap(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int box_rows);
-int env_int(const char* name, int dflt);
 
 // Scratch of one fused call: arena_begin sizes the (device, stream) block for the whole call, arena_take carves it.
 struct ArenaCursor {

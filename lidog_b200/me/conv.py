@@ -31,7 +31,6 @@ CONFIG = {
     # (lg_prep_weights + lg_conv_gemm_tc + lg_conv_wgrad_tc, workspaces from torch) kept for A/B runs
     "layer_calls": int(os.environ.get("LIDOG_LAYER_CALLS", "1")),
 }
-GATHER_MODE = 2  # the only pipeline in the library (include/lidog_b200.h, lg_conv_gemm_tc)
 
 
 # Instrumentation for bench.py / tools (never on in a timed headline loop): per-launch CUDA events + algorithmic FLOPs
@@ -89,7 +88,7 @@ def _gemm_tc(plan, A16, B16, N, flip, fmt, out_scale, bias):
 
     def launch():
         cabi.check(cabi.lib().lg_conv_gemm_tc(plan.cref, cabi.ptr(A16), A16.shape[1], cabi.ptr(B16), N, flip, fmt,
-                                              cabi.ptr(out_scale), cabi.ptr(bias), cabi.ptr(Y), GATHER_MODE,
+                                              cabi.ptr(out_scale), cabi.ptr(bias), cabi.ptr(Y),
                                               cabi.stream_of(A16)), "lg_conv_gemm_tc")
     if PROFILE["enabled"]:
         _profiled("k_gemm_tc", plan, A16.shape[1], N, launch)
@@ -222,7 +221,7 @@ class SparseConvFunction(torch.autograd.Function):
 
                     def launch():
                         cabi.check(L.lg_conv_wgrad_tc(p_wgrad.cref, cabi.ptr(x16), cin, cabi.ptr(dy16), cout, fmt,
-                                                      cabi.ptr(inv), cabi.ptr(dw), GATHER_MODE, cabi.ptr(ws), ws_bytes,
+                                                      cabi.ptr(inv), cabi.ptr(dw), cabi.ptr(ws), ws_bytes,
                                                       cabi.stream_of(dy)), "lg_conv_wgrad_tc")
                     if PROFILE["enabled"]:
                         _profiled("k_wgrad_tc", p_wgrad, cin, cout, launch)

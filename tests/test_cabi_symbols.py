@@ -57,6 +57,16 @@ def test_sass_contains_blackwell_tensor_and_tma_instructions(libpath):
         assert mnemonic in sass, mnemonic
     # the first-generation gather4 kernels are not in the product library any more
     assert "GATHER4" not in sass
+    # nor is the L2 row prefetch of k_gemm2 (cp.async.bulk.prefetch.L2: measured slower than the LDGSTS gathers)
+    assert "UBLKPF" not in sass
+
+
+def test_library_reads_no_environment():
+    """The native library's behaviour depends on its arguments only: no source under csrc/ reads the environment."""
+    csrc = os.path.join(ROOT, "lidog_b200", "csrc")
+    for name in sorted(os.listdir(csrc)):
+        src = open(os.path.join(csrc, name)).read()
+        assert not re.search(r"\bgetenv\b", src), name
 
 
 def test_minkowski_engine_surface_matches_reference_usage():
@@ -119,12 +129,9 @@ def test_model_state_dict_matches_reference_names():
 def test_wgrad_workspace_covers_the_chunk_rule(libpath):
     """`lg_conv_wgrad_tc_workspace` is host-only and must cover the partial-dW buffers of `k_wgrad2`:
     chunks x K x Cin x Cout floats, chunks = tiles / 32 clamped to [one wave of 148 CTAs, four waves] over the
-    (offset group x 128-channel block) CTAs (csrc/conv_tc2.cu, from the CTA sweep in profiles/r01_s4_sweep_a.txt).
-    (The entry point returns the maximum over the kernel generations, so this is a lower bound.)"""
+    (offset group x 128-channel block) CTAs (csrc/conv_tc2.cu, from the CTA sweep in profiles/r01_s4_sweep_a.txt)."""
     import math
-    import os
     from lidog_b200 import cabi
-    os.environ.pop("LIDOG_WG_CTAS", None)
     L = cabi.lib()
 
     def workspace(n_tiles, K, cin, cout):

@@ -49,7 +49,6 @@ def main():
     ap.add_argument("--fmt", default="fp16")
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--cases", default="all")
-    ap.add_argument("--gather", default="2")
     ap.add_argument("--only", default="fwd,dgrad,wgrad")
     ap.add_argument("--sorted", default="0,1", help="gather-plan row order: 0 natural, 1 mask-sorted")
     ap.add_argument("--points", type=int, default=0,
@@ -96,28 +95,27 @@ def main():
           dw = torch.empty(K, cin, cout, device=dev)
           ws_bytes = L.lg_conv_wgrad_tc_workspace(p_wgrad.c, cin, cout)
           ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-          for gather in [int(g) for g in args.gather.split(",")]:
-              res = {}
-              if "fwd" in only:
-                  res["fwd"] = (timed(lambda: cabi.check(L.lg_conv_gemm_tc(
-                      p_fwd.c, cabi.ptr(x16), cin, cabi.ptr(w16t), cout, 0, fmt, None, None, cabi.ptr(y), gather,
-                      cabi.stream())), args.reps), units, cin, cout)
-              if "dgrad" in only:
-                  res["dgrad"] = (timed(lambda: cabi.check(L.lg_conv_gemm_tc(
-                      p_dgrad.c, cabi.ptr(dy16), cout, cabi.ptr(w16), cin, flip, fmt, None, None, cabi.ptr(dx), gather,
-                      cabi.stream())), args.reps), units_d, cout, cin)
-              if "wgrad" in only:
-                  res["wgrad"] = (timed(lambda: cabi.check(L.lg_conv_wgrad_tc(
-                      p_wgrad.c, cabi.ptr(x16), cin, cabi.ptr(dy16), cout, fmt, None, cabi.ptr(dw), gather, cabi.ptr(ws),
-                      ws_bytes, cabi.stream())), args.reps), units, cin, cout)
-              for name, (ms, u, a, b) in res.items():
-                  alg = 2.0 * pairs * cin * cout / (ms * 1e-3) / 1e12
-                  dense = 2.0 * u * 128 * cin * cout / (ms * 1e-3) / 1e12
-                  cyc = ms * 1e-3 * clock_mhz * 1e6 * sm_count / max(u, 1)
-                  print(json.dumps(dict(case=f"{kind} ts{ts} k{ks} {cin}->{cout}", op=name, gather=gather, sorted=srt, ms=round(ms, 4),
-                                        n_out=p_fwd.n_out, pairs=pairs, units=u, density=round(pairs / max(u * 128, 1), 3),
-                                        alg_tflops=round(alg, 1), dense_tflops=round(dense, 1),
-                                        sm_cycles_per_unit=round(cyc))), flush=True)
+          res = {}
+          if "fwd" in only:
+              res["fwd"] = (timed(lambda: cabi.check(L.lg_conv_gemm_tc(
+                  p_fwd.c, cabi.ptr(x16), cin, cabi.ptr(w16t), cout, 0, fmt, None, None, cabi.ptr(y),
+                  cabi.stream())), args.reps), units, cin, cout)
+          if "dgrad" in only:
+              res["dgrad"] = (timed(lambda: cabi.check(L.lg_conv_gemm_tc(
+                  p_dgrad.c, cabi.ptr(dy16), cout, cabi.ptr(w16), cin, flip, fmt, None, None, cabi.ptr(dx),
+                  cabi.stream())), args.reps), units_d, cout, cin)
+          if "wgrad" in only:
+              res["wgrad"] = (timed(lambda: cabi.check(L.lg_conv_wgrad_tc(
+                  p_wgrad.c, cabi.ptr(x16), cin, cabi.ptr(dy16), cout, fmt, None, cabi.ptr(dw), cabi.ptr(ws),
+                  ws_bytes, cabi.stream())), args.reps), units, cin, cout)
+          for name, (ms, u, a, b) in res.items():
+              alg = 2.0 * pairs * cin * cout / (ms * 1e-3) / 1e12
+              dense = 2.0 * u * 128 * cin * cout / (ms * 1e-3) / 1e12
+              cyc = ms * 1e-3 * clock_mhz * 1e6 * sm_count / max(u, 1)
+              print(json.dumps(dict(case=f"{kind} ts{ts} k{ks} {cin}->{cout}", op=name, sorted=srt, ms=round(ms, 4),
+                                    n_out=p_fwd.n_out, pairs=pairs, units=u, density=round(pairs / max(u * 128, 1), 3),
+                                    alg_tflops=round(alg, 1), dense_tflops=round(dense, 1),
+                                    sm_cycles_per_unit=round(cyc))), flush=True)
 
 
 if __name__ == "__main__":

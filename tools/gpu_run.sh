@@ -81,8 +81,6 @@ for step in "$@"; do
               done ;;
     tests_syncbn) timeout 900 python -m pytest tests/test_gpu_syncbn.py -m gpu -q 2>&1 | tail -5 | tee ${O}_tests_syncbn.log ;;
     sanitize) bash tools/sanitize.sh ${O} ;;
-    wgdiag)   bash tools/wgrad_diag.sh 2>&1 | tee ${O}_wgrad_diag.txt | tail -30 ;;
-    bisect)   bash tools/bisect_wgrad.sh 2>&1 | tee ${O}_bisect.log ;;
     *) echo "unknown step $step" ;;
   esac
 done
