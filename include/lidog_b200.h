@@ -220,6 +220,14 @@ int lg_conv_layer_forward(const lgConvPlan* plan, const void* X16, int32_t Cin, 
 int lg_conv_layer_backward(const lgConvPlan* plan_dgrad, const lgConvPlan* plan_wgrad, int32_t flip_dgrad,
                            const void* X16, int32_t Cin, const void* dY16, int32_t Cout, const void* w16, int32_t fmt,
                            const float* inv_scale, float* dX, float* dW, void* stream);
+/* MinkowskiConvolution -> MinkowskiBatchNorm (eval: running statistics) [-> += residual] [-> MinkowskiReLU] in one
+ * launch.  bn_stats float[4C] in the lg_bn_apply layout ([mean, invstd, scale, shift]; only scale / shift are read).
+ * res nullable fp32 [n_out, Cout]; Y fp32 required; Y16 nullable.  Cout column blocks must be multiples of 32.
+ * W, w16, w16t, prep, fmt as lg_conv_layer_forward; no bias (no tensor-core layer before a batch norm has one).
+ * Y and Y16 are bit-identical to lg_conv_layer_forward followed by lg_bn_apply(Y, bn_stats, res, relu). */
+int lg_conv_layer_infer(const lgConvPlan* plan, const void* X16, int32_t Cin, const float* W, int32_t Cout, void* w16,
+                        void* w16t, int32_t prep, int32_t fmt, const float* bn_stats, const float* res, int32_t relu,
+                        float* Y, void* Y16, void* stream);
 
 /* Library-owned scratch arena (one block per device and stream, outside any caching allocator): bytes currently held,
  * and release (synchronises).  The layer-level calls size it themselves. */
@@ -336,6 +344,14 @@ int lg_dice_forward(const float* logits, const int64_t* target, int64_t n, int32
 int lg_dice_backward(const float* logits, const int64_t* target, int64_t n, int32_t C, int32_t ignore_label,
                      int32_t soft, float eps, int32_t is_kitti, const float* coef, const float* grad_scale,
                      float* dlogits, void* stream);
+
+/* ------------------------------------------------------------------ evaluation metric
+ *
+ * ADDS the confusion matrix of one batch into conf int64 [(C + 1) x C]: row = target class, row C = every target
+ * outside [0, C) (the ignore label included), column = argmax_c logits[i, c] (first maximal index, torch's rule).
+ * logits float [n, C] (1 <= C <= 32), target int64 [n].  n = 0 does nothing.  Exact and run-to-run identical.
+ * IoU as torchmetrics JaccardIndex(ignore_index): rows 0..C-1; as sklearn jaccard_score(labels=range(C)): all rows. */
+int lg_confusion_matrix(const float* logits, int64_t n, int32_t C, const int64_t* target, int64_t* conf, void* stream);
 
 /* ------------------------------------------------------------------ BEV projection */
 

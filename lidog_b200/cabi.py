@@ -79,6 +79,8 @@ SIGNATURES = {
     "lg_conv_wgrad_tc": (C.c_int, [_PP, _vp, _i32, _vp, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
     "lg_conv_layer_forward": (C.c_int, [_PP, _vp, _i32, _vp, _i32, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp]),
     "lg_conv_layer_backward": (C.c_int, [_PP, _PP, _i32, _vp, _i32, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _vp]),
+    "lg_conv_layer_infer": (C.c_int, [_PP, _vp, _i32, _vp, _i32, _vp, _vp, _i32, _i32, _vp, _vp, _i32, _vp, _vp, _vp]),
+    "lg_confusion_matrix": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _vp]),
     "lg_arena_bytes": (_sz, []),
     "lg_arena_release": (C.c_int, []),
     "lg_bn_layer_forward": (C.c_int, [_PB, _PB, _vp, _i32, _i64, _i32, _vp, _vp, _i32, _PPC, _vp]),
@@ -115,6 +117,8 @@ KERNELS_PER_CALL = {
     "lg_bn_stats": 2, "lg_bn_finalize": 1, "lg_bn_apply": 1, "lg_bn_bwd_stats": 2, "lg_bn_bwd_finalize": 1,
     "lg_bn_bwd_gscale": 1, "lg_bn_bwd_apply": 1, "lg_peer_sum": 1,
     "lg_bn_layer_backward": 3, "lg_dice_forward": 2, "lg_dice_backward": 1,
+    # + 1 (lg_prep_weights) when the call refreshes the 16-bit weights: counted by the caller
+    "lg_conv_layer_infer": 1, "lg_confusion_matrix": 1,
 }
 COUNTS: dict = {}
 _RAW = None

@@ -17,6 +17,10 @@
 // Shared-memory operand tiles use the SWIZZLE_64B layout (64-byte rows = 32 channels).
 // Results are deterministic: every output row / weight element is written once in a fixed order.
 // Reference contract: MinkowskiConvolution(+Transpose) forward/backward, utils/models/minkunet_bev.py:57-123.
+// Inference (k_gemm2<PC, true>): the epilogue also applies the eval-mode batch norm, the residual and the ReLU that
+// follow the convolution, with k_bn_apply's expression, and writes the 16-bit operand copy (lg_conv_layer_infer).
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -197,10 +201,75 @@ struct Gemm2Args {
   int* sched;  // [0..3] next super-tile per blockIdx.y, [4] finished CTAs (self-resetting)
 };
 
+// Epilogue of the inference instantiations: Y = act(fmaf(acc, scale, shift) [+ res]), Y16 = 16-bit copy of Y.
+// A separate kernel parameter after the tensor map, so the training instantiations keep their parameter layout.
+struct InferEpi {
+  const float* scale;  // [N] = bn_stats + 2N (lg_bn_apply layout)
+  const float* shift;  // [N] = bn_stats + 3N
+  const float* res;    // nullable [n_out][N]
+  uint16_t* Y16;       // nullable [n_out][N]
+  int relu, fmt;
+};
+
+// same rounding as bn_to16 (bn.cu): the 16-bit copy equals the one lg_bn_apply writes
+__device__ __forceinline__ uint16_t epi_to16(float v, int fmt) {
+  if (fmt == LG_FMT_BF16) return __bfloat16_as_ushort(__float2bfloat16_rn(v));
+  v = fminf(fmaxf(v, -65504.f), 65504.f);
+  return __half_as_ushort(__float2half_rn(v));
+}
+
+// One 32-column block of 32 rows of the inference epilogue.  Lane = (row (lane >> 3) + 4 j, columns 4 (lane & 7)..+3):
+// every warp instruction reads / writes 4 rows x 128 contiguous bytes (Y, res) or 4 x 64 bytes (Y16), like the staged
+// Y store of the training epilogue.  `stg` holds the accumulators transposed through shared memory, or nothing when
+// the tile has no neighbour at all (acc = 0: fmaf(0, s, h) is what k_bn_apply computes on the zeros the training
+// epilogue writes there).  The expression is k_bn_apply's, operation by operation, so the result is bit-identical
+// to lg_conv_layer_forward followed by lg_bn_apply.
+// The loads (scale, shift, the 8 residual rows) are issued by infer_loads before the accumulators are read from TMEM:
+// the compiler cannot move them above the stores to Y (res and Y may alias as far as it knows), so loaded inside the
+// row loop each row would wait for its own residual load in series.
+struct InferIn {
+  float4 sc, sh, r[8];
+};
+__device__ __forceinline__ void infer_loads(const InferEpi& e, InferIn& in, const int (&srow)[8], int N, int c) {
+  in.sc = __ldg(reinterpret_cast<const float4*>(e.scale + c));
+  in.sh = __ldg(reinterpret_cast<const float4*>(e.shift + c));
+  if (e.res) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j)
+      if (srow[j] >= 0) in.r[j] = __ldg(reinterpret_cast<const float4*>(e.res + (int64_t)srow[j] * N + c));
+  }
+}
+__device__ __forceinline__ void infer_block(const InferEpi& e, const InferIn& in, const float* stg, bool have,
+                                            const int (&srow)[8], float* Y, int N, int c, int lane) {
+  const float4 sc = in.sc, sh = in.sh;
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    if (srow[j] < 0) continue;
+    const int64_t off = (int64_t)srow[j] * N + c;
+    float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (have) a = *reinterpret_cast<const float4*>(stg + ((lane >> 3) + 4 * j) * kStgPitch + 4 * (lane & 7));
+    float4 o = make_float4(fmaf(a.x, sc.x, sh.x), fmaf(a.y, sc.y, sh.y), fmaf(a.z, sc.z, sh.z), fmaf(a.w, sc.w, sh.w));
+    if (e.res) {
+      const float4 r = in.r[j];
+      o.x += r.x, o.y += r.y, o.z += r.z, o.w += r.w;
+    }
+    if (e.relu) o = make_float4(fmaxf(o.x, 0.f), fmaxf(o.y, 0.f), fmaxf(o.z, 0.f), fmaxf(o.w, 0.f));
+    *reinterpret_cast<float4*>(Y + off) = o;
+    if (e.Y16) {
+      uint2 h;
+      h.x = epi_to16(o.x, e.fmt) | ((uint32_t)epi_to16(o.y, e.fmt) << 16);
+      h.y = epi_to16(o.z, e.fmt) | ((uint32_t)epi_to16(o.w, e.fmt) << 16);
+      *reinterpret_cast<uint2*>(e.Y16 + off) = h;
+    }
+  }
+}
+
 // PC: 32-channel chunks per operand stage (= g.pc).  TMEM holds two accumulator sets of T tiles (2 * T * n_blk <= 512
 // columns): the epilogue of one super-tile overlaps the MMAs of the next.
-template <int PC>
-__global__ void __launch_bounds__(kThreads, 1) k_gemm2(const Gemm2Args g, const __grid_constant__ CUtensorMap tmB) {
+// INFER: the inference epilogue (InferEpi; no statistics, no bias, no out_scale, n_blk % 32 == 0 -- host-checked).
+template <int PC, bool INFER>
+__global__ void __launch_bounds__(kThreads, 1)
+    k_gemm2(const Gemm2Args g, const __grid_constant__ CUtensorMap tmB, const InferEpi e) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -493,6 +562,37 @@ __global__ void __launch_bounds__(kThreads, 1) k_gemm2(const Gemm2Args g, const 
           const int64_t s = (tile0 + t) * LG_TILE_ROWS + warp * 32 + lane;
           int64_t row = g.plan.out_row ? (int64_t)g.plan.out_row[s] : s;
           const bool row_ok = row >= 0 && row < g.plan.n_out;
+          if constexpr (INFER) {
+            const bool have = (am >> t) & 1u;
+            const uint32_t taddr = tmem_base + (a0 + t) * g.n_blk + ((uint32_t)(warp * 32) << 16);
+            float* stg = smStg + warp * 32 * kStgPitch;
+            int srow[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j) srow[j] = __shfl_sync(0xffffffffu, row_ok ? (int)row : -1, (lane >> 3) + 4 * j);
+            for (int n = 0; n < g.n_blk; n += 32) {
+              const int c = n0 + n + 4 * (lane & 7);
+              InferIn in;
+              infer_loads(e, in, srow, g.N, c);
+              if (have) {
+                uint32_t v[32];
+                tmem_ld32(taddr + n, v);
+                tmem_ld_wait();
+#pragma unroll
+                for (int q = 0; q < 8; ++q)
+                  *reinterpret_cast<float4*>(stg + lane * kStgPitch + 4 * q) =
+                      make_float4(__uint_as_float(v[4 * q + 0]), __uint_as_float(v[4 * q + 1]),
+                                  __uint_as_float(v[4 * q + 2]), __uint_as_float(v[4 * q + 3]));
+                __syncwarp();
+              }
+              infer_block(e, in, stg, have, srow, g.Y, g.N, c, lane);
+              __syncwarp();
+            }
+            if (am) {  // hand accumulator t back
+              tc_fence_before();
+              mbar_arrive(&acc_empty[a0 + t]);
+            }
+            continue;
+          }
           float* yrow = g.Y + (row_ok ? row : 0) * g.N + n0;
           // BN statistics of the layer that follows (SURVEY.md 8f-1): this warp's 32 rows contribute one partial
           // row [sum | sum of squares] per tile; a fixed shuffle order and a fixed (tile, warp) slot keep the later
@@ -931,9 +1031,12 @@ struct Gemm2Shape {
   size_t smem;
 };
 
+// column-block width of k_gemm2 for N output columns (blocks of <= 256 columns, equal widths)
+static inline int gemm2_n_blk(int N) { return N / ((N + 255) / 256); }
+
 static int gemm2_shape(int64_t n_tiles, int Ck, int N, int sm_count, bool stats, Gemm2Shape* s) {
   s->n_split = (N + 255) / 256;
-  s->n_blk = N / s->n_split;
+  s->n_blk = gemm2_n_blk(N);
   if (s->n_blk % 16 != 0 || s->n_blk * s->n_split != N) {
     set_error("lg_conv_gemm_tc: N=%d cannot be split into equal multiples of 16", N);
     return LG_ERR_UNSUPPORTED;
@@ -997,9 +1100,14 @@ static int gemm2_shape(int64_t n_tiles, int Ck, int N, int sm_count, bool stats,
 }  // namespace v2
 
 // host launcher: forward / dgrad
+// infer (nullable): run the inference epilogue (k_gemm2<PC, true>); out_scale, bias and stats must then be null
 int launch_gemm_tc2(const lgConvPlan* plan, const void* A16, int Ck, const void* B16, int N, int flip_k, int fmt,
-                    const float* out_scale, const float* bias, float* Y, float* stats, cudaStream_t stream) {
+                    const float* out_scale, const float* bias, float* Y, float* stats, cudaStream_t stream,
+                    const v2::InferEpi* infer = nullptr) {
   using namespace v2;
+  // the inference epilogue has no bias, no output scale and no statistics, and no 16-column remainder path
+  LG_CHECK_ARG(!infer || (!out_scale && !bias && !stats && gemm2_n_blk(N) % 32 == 0),
+               "launch_gemm_tc2: the inference epilogue takes no bias / out_scale / statistics and 32-column blocks");
   int sm_count = 0;
   int* err = nullptr;
   int rc = tc_runtime(&sm_count, &err);
@@ -1037,16 +1145,28 @@ int launch_gemm_tc2(const lgConvPlan* plan, const void* A16, int Ck, const void*
   if (rc) return rc;
   const dim3 grid((unsigned)(s.n_super < sm_count ? s.n_super : sm_count), (unsigned)s.n_split);
   const size_t smem = s.smem;
-#define LG_LAUNCH_GEMM2(PCV)                                                                                   \
-  do {                                                                                                         \
-    LG_CUDA_OK(cudaFuncSetAttribute(k_gemm2<PCV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
-    k_gemm2<PCV><<<grid, kThreads, smem, stream>>>(g, tmB);                                                    \
+  InferEpi e;
+  memset(&e, 0, sizeof(e));
+  if (infer) e = *infer;
+#define LG_LAUNCH_GEMM2(PCV, INF)                                                                                 \
+  do {                                                                                                            \
+    LG_CUDA_OK(cudaFuncSetAttribute(k_gemm2<PCV, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));  \
+    k_gemm2<PCV, INF><<<grid, kThreads, smem, stream>>>(g, tmB, e);                                               \
   } while (0)
-  switch (g.pc) {
-    case 1: LG_LAUNCH_GEMM2(1); break;
-    case 2: LG_LAUNCH_GEMM2(2); break;
-    case 3: LG_LAUNCH_GEMM2(3); break;
-    default: LG_LAUNCH_GEMM2(4); break;
+  if (infer) {
+    switch (g.pc) {
+      case 1: LG_LAUNCH_GEMM2(1, true); break;
+      case 2: LG_LAUNCH_GEMM2(2, true); break;
+      case 3: LG_LAUNCH_GEMM2(3, true); break;
+      default: LG_LAUNCH_GEMM2(4, true); break;
+    }
+  } else {
+    switch (g.pc) {
+      case 1: LG_LAUNCH_GEMM2(1, false); break;
+      case 2: LG_LAUNCH_GEMM2(2, false); break;
+      case 3: LG_LAUNCH_GEMM2(3, false); break;
+      default: LG_LAUNCH_GEMM2(4, false); break;
+    }
   }
 #undef LG_LAUNCH_GEMM2
   LG_LAUNCH_OK();
@@ -1219,6 +1339,35 @@ extern "C" int lg_conv_layer_forward(const lgConvPlan* plan, const void* X16, in
     if (rc) return rc;
   }
   return launch_gemm_tc2(plan, X16, Cin, w16t, Cout, 0, fmt, nullptr, bias, Y, stat_partials, (cudaStream_t)stream_);
+}
+
+/* Inference form of lg_conv_layer_forward: convolution -> eval-mode batch norm [-> + res] [-> ReLU] in one launch
+ * (see include/lidog_b200.h). */
+extern "C" int lg_conv_layer_infer(const lgConvPlan* plan, const void* X16, int32_t Cin, const float* W, int32_t Cout,
+                                   void* w16, void* w16t, int32_t prep, int32_t fmt, const float* bn_stats,
+                                   const float* res, int32_t relu, float* Y, void* Y16, void* stream_) {
+  int rc = check_gemm(plan, Cin, Cout, fmt, "lg_conv_layer_infer");
+  if (rc) return rc;
+  LG_CHECK_ARG(X16 && w16t && Y && bn_stats && (!prep || (W && w16)), "lg_conv_layer_infer: null pointer");
+  const auto misaligned = [](const void* p, uintptr_t a) { return ((uintptr_t)p & (a - 1)) != 0; };
+  LG_CHECK_ARG(!misaligned(Y, 16) && !misaligned(bn_stats, 16) && !misaligned(res, 16) && !misaligned(Y16, 8),
+               "lg_conv_layer_infer: Y, bn_stats and res must be 16-byte aligned, Y16 8-byte aligned");
+  if (v2::gemm2_n_blk(Cout) % 32 != 0) {
+    set_error("lg_conv_layer_infer: Cout=%d gives column blocks that are not multiples of 32", Cout);
+    return LG_ERR_UNSUPPORTED;
+  }
+  if (prep) {
+    rc = lg_prep_weights(W, plan->kernel_volume, Cin, Cout, w16, w16t, fmt, stream_);
+    if (rc) return rc;
+  }
+  v2::InferEpi e;
+  e.scale = bn_stats + 2 * Cout;
+  e.shift = bn_stats + 3 * Cout;
+  e.res = res;
+  e.Y16 = (uint16_t*)Y16;
+  e.relu = relu ? 1 : 0;
+  e.fmt = fmt;
+  return launch_gemm_tc2(plan, X16, Cin, w16t, Cout, 0, fmt, nullptr, nullptr, Y, nullptr, (cudaStream_t)stream_, &e);
 }
 
 /* dgrad and wgrad of one MinkowskiConvolution in one host call; the split-K partials live in the library arena. */

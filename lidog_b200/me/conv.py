@@ -302,6 +302,9 @@ class MinkowskiConvolutionBase(nn.Module):
         assert isinstance(input, SparseTensor)
         cm = input.coordinate_manager
         ts_out, plans = self._plans(cm, input._ts)
+        if not self.training and infer_fast_path(False, torch.is_grad_enabled(), self.bias is not None,
+                                                 self.in_channels, self.out_channels, input.F.is_cuda, plans[0].n_out):
+            return DeferredConv(self, input, plans, ts_out)
         box = {} if self.training else None
         y = SparseConvFunction.apply(input.F, self.kernel, self.bias, plans, input, self._wcache, box)
         out = SparseTensor(y, tensor_stride=ts_out, coordinate_manager=cm)
@@ -309,9 +312,97 @@ class MinkowskiConvolutionBase(nn.Module):
             out._stat_partials = (box["stats"], y._version)
         return out
 
+    def _forward_now(self, input: SparseTensor, plans, ts_out) -> SparseTensor:
+        """Today's forward of an eval-mode layer: the convolution alone (no epilogue statistics)."""
+        y = SparseConvFunction.apply(input.F, self.kernel, self.bias, plans, input, self._wcache, None)
+        return SparseTensor(y, tensor_stride=ts_out, coordinate_manager=input.coordinate_manager)
+
     def __repr__(self):
         return (f"{self.__class__.__name__}(in={self.in_channels}, out={self.out_channels}, "
                 f"kernel_size={[self.kernel_size] * 3}, stride={[self.stride] * 3}, dilation=[1, 1, 1])")
+
+
+def infer_fast_path(training, grad_enabled, has_bias, cin, cout, is_cuda, n_out) -> bool:
+    """Whether a convolution forward returns a DeferredConv (inference epilogue, lg_conv_layer_infer): only in eval mode
+    without autograd, on the tensor-core path with one library call per layer and no instrumentation, for a layer
+    without bias whose column blocks are multiples of 32, on a non-empty output.  Everything else runs the forward of
+    training and of eval with gradients unchanged."""
+    return (not training and not grad_enabled and not has_bias and _tc_ok(cin, cout)
+            and (cout // ((cout + 255) // 256)) % 32 == 0 and bool(CONFIG["layer_calls"]) and not PROFILE["enabled"]
+            and is_cuda and n_out > 0)
+
+
+class DeferredConv(SparseTensor):
+    """Output of an eval-mode tensor-core convolution that has not been launched yet (the inference counterpart of
+    me/norm.py's DeferredBN, one step earlier).  An eval-mode MinkowskiBatchNorm attaches its running-statistics
+    coefficients, `+=` a residual, and MinkowskiReLU launches conv -> BN [-> + residual] -> ReLU as ONE library call
+    that also writes the 16-bit operand copy of the next convolution.  Any other read of `.F` launches without ReLU
+    (and without anything, when no batch norm was attached: the plain convolution)."""
+
+    def __init__(self, conv: MinkowskiConvolutionBase, src: SparseTensor, plans, ts_out: int):
+        self.coordinate_manager = src.coordinate_manager
+        self._ts = ts_out
+        self._f16_cache = None
+        self._conv, self._src, self._plans = conv, src, plans
+        self._bn_stats = None   # float32 [4 * Cout] in the lg_bn_apply layout, set by MinkowskiBatchNorm
+        self._residual = None   # fp32 [n_out, Cout] features of the residual, set by +=
+        self._value = None
+
+    @property
+    def _F(self):
+        if self._value is None:
+            self._launch(False)
+        return self._value
+
+    @_F.setter
+    def _F(self, v):
+        self._value = v
+
+    def accepts_bn(self, num_features: int) -> bool:
+        """A batch norm of `num_features` channels can still be attached: not launched, nothing attached yet."""
+        return (self._value is None and self._bn_stats is None and self._residual is None
+                and num_features == self._conv.out_channels)
+
+    def __iadd__(self, other):
+        if self._value is None and self._bn_stats is not None and self._residual is None and isinstance(other, SparseTensor):
+            self._same_map(other)
+            if isinstance(other, DeferredConv) and other._value is None:
+                other._launch(False)  # the block's downsample (1x1 conv + BN): launched first, without ReLU
+            r = other.F
+            if (r.dtype == torch.float32 and r.is_contiguous() and r.data_ptr() % 16 == 0
+                    and tuple(r.shape) == (self._plans[0].n_out, self._conv.out_channels)):
+                self._residual = r
+                return self
+        return SparseTensor.__iadd__(self, other)
+
+    def _launch(self, relu: bool):
+        conv, src = self._conv, self._src
+        if self._bn_stats is None:  # nothing to fuse: the plain convolution
+            self._value = conv._forward_now(src, self._plans, self._ts).F
+            self._src = None
+            return self
+        p = self._plans[0]
+        kernel = conv.kernel.detach()
+        if kernel.dim() == 3:
+            K, cin, cout = kernel.shape
+        else:
+            K, (cin, cout) = 1, kernel.shape
+        fmt = _fmt()
+        x16 = src._f16(fmt)
+        Wc = kernel if kernel.is_contiguous() else kernel.contiguous()
+        w16, w16t, stale = conv._wcache.get(Wc, K, cin, cout, fmt)
+        res = self._residual
+        y = torch.empty((p.n_out, cout), dtype=torch.float32, device=x16.device)
+        y16 = torch.empty((p.n_out, cout), dtype=_dt16(fmt), device=x16.device)
+        cabi.check(cabi.lib().lg_conv_layer_infer(p.cref, x16.data_ptr(), cin, Wc.data_ptr(), cout, w16.data_ptr(),
+                                                  w16t.data_ptr(), 1 if stale else 0, fmt, self._bn_stats.data_ptr(),
+                                                  cabi.ptr(res), 1 if relu else 0, y.data_ptr(), y16.data_ptr(),
+                                                  cabi.stream_of(y)), "lg_conv_layer_infer")
+        cabi.count_launches("lg_conv_layer_infer", 1 if stale else 0)
+        self._value = y
+        self._f16_cache = ((fmt, y._version, y.data_ptr()), y16)  # the next convolution's operand: no cast pass
+        self._src = self._residual = self._bn_stats = None
+        return self
 
 
 class MinkowskiConvolution(MinkowskiConvolutionBase):

@@ -28,6 +28,7 @@ import torch
 import torch.nn as nn
 
 from .. import cabi
+from .conv import DeferredConv
 from .sparse_tensor import SparseTensor
 
 import ctypes as _C
@@ -393,6 +394,25 @@ class DeferredBN(SparseTensor):
         return SparseTensor.__iadd__(self, other)
 
 
+def eval_bn_stats(bn) -> torch.Tensor:
+    """Eval-mode coefficients of a BatchNorm1d in the lg_bn_apply layout, float32 [4C] = [mean, invstd, scale, shift]:
+    scale = gamma / sqrt(running_var + eps), shift = beta - running_mean * scale, computed in float64 and rounded once."""
+    mean, var = bn.running_mean.detach().double(), bn.running_var.detach().double()
+    std = torch.sqrt(var + bn.eps)
+    invstd = 1.0 / std
+    scale = bn.weight.detach().double() / std if bn.affine else invstd
+    shift = -mean * scale
+    if bn.affine:
+        shift = shift + bn.bias.detach().double()
+    return torch.cat([mean, invstd, scale, shift]).float().contiguous()
+
+
+def _infer_attachable(bn) -> bool:
+    """An eval-mode BN that normalises with its running statistics can join the preceding convolution's launch."""
+    return (not bn.training and bn.track_running_stats and bn.running_mean is not None
+            and bn.running_var is not None)
+
+
 class MinkowskiBatchNorm(nn.Module):
     def __init__(self, num_features, eps=1e-5, momentum=0.1, affine=True, track_running_stats=True):
         super().__init__()
@@ -400,9 +420,30 @@ class MinkowskiBatchNorm(nn.Module):
                                  track_running_stats=track_running_stats)
 
     def forward(self, input: SparseTensor) -> SparseTensor:
+        if isinstance(input, DeferredConv) and _infer_attachable(self.bn) and input.accepts_bn(self.bn.num_features):
+            input._bn_stats = self._eval_stats()
+            return input
         if _fusable(self.bn, input.F):
             return DeferredBN(input, self.bn)
         return input._like(self.bn(input.F))
+
+    def _eval_stats(self) -> torch.Tensor:
+        """eval_bn_stats(self.bn), cached until a parameter or buffer is replaced or modified by torch, or the module
+        goes back to training mode (the training kernels update the running buffers in place, invisibly to
+        `_version`)."""
+        b = self.bn
+        key = tuple((t._version, t.data_ptr()) for t in (b.weight, b.bias, b.running_mean, b.running_var)
+                    if t is not None)
+        cache = self.__dict__.get("_eval_cache")
+        if cache is None or cache[0] != key:
+            cache = (key, eval_bn_stats(b))
+            self.__dict__["_eval_cache"] = cache
+        return cache[1]
+
+    def train(self, mode: bool = True):
+        if mode:  # running statistics change only in training mode
+            self.__dict__.pop("_eval_cache", None)
+        return super().train(mode)
 
     def __repr__(self):
         b = self.bn
@@ -444,6 +485,8 @@ class MinkowskiReLU(nn.Module):
     def forward(self, input: SparseTensor) -> SparseTensor:
         if isinstance(input, DeferredBN) and input._value is None:
             return input._evaluate(True)
+        if isinstance(input, DeferredConv) and input._value is None and input._bn_stats is not None:
+            return input._launch(True)
         return input._like(torch.relu_(input.F) if self.inplace else torch.relu(input.F))
 
 
