@@ -60,8 +60,15 @@ def _fmt():
     return {"fp16": cabi.FMT_FP16, "bf16": cabi.FMT_BF16}.get(CONFIG["tc"])
 
 
-def _tc_ok(cin, cout):
-    return _fmt() is not None and cin % 32 == 0 and cout % 32 == 0
+# The tensor-core wgrad (k_wgrad2) takes at most 64 kernel offsets (two mask words); a layer with more (kernel size 5:
+# 125 offsets) runs forward and backward on the SIMT kernels.  The whole layer moves: the tensor-core forward keeps only
+# the 16-bit copy of x, and the SIMT wgrad needs the fp32 x.
+TC_MAX_KERNEL_VOLUME = 64
+
+
+def _tc_ok(cin, cout, kernel_volume):
+    return (_fmt() is not None and cin % 32 == 0 and cout % 32 == 0
+            and kernel_volume <= TC_MAX_KERNEL_VOLUME)
 
 
 def _dt16(fmt):
@@ -136,7 +143,7 @@ class SparseConvFunction(torch.autograd.Function):
         x = x.contiguous()
         ctx.plans, ctx.shape, ctx.kdim = plans, (K, cin, cout), kernel.dim()
         ctx.has_bias = bias is not None
-        ctx.tc = _tc_ok(cin, cout) and x.shape[0] > 0
+        ctx.tc = _tc_ok(cin, cout, K) and x.shape[0] > 0
         L = cabi.lib()
         if ctx.tc:
             fmt = _fmt()
@@ -303,7 +310,8 @@ class MinkowskiConvolutionBase(nn.Module):
         cm = input.coordinate_manager
         ts_out, plans = self._plans(cm, input._ts)
         if not self.training and infer_fast_path(False, torch.is_grad_enabled(), self.bias is not None,
-                                                 self.in_channels, self.out_channels, input.F.is_cuda, plans[0].n_out):
+                                                 self.in_channels, self.out_channels, input.F.is_cuda, plans[0].n_out,
+                                                 self.kernel_volume):
             return DeferredConv(self, input, plans, ts_out)
         box = {} if self.training else None
         y = SparseConvFunction.apply(input.F, self.kernel, self.bias, plans, input, self._wcache, box)
@@ -322,12 +330,12 @@ class MinkowskiConvolutionBase(nn.Module):
                 f"kernel_size={[self.kernel_size] * 3}, stride={[self.stride] * 3}, dilation=[1, 1, 1])")
 
 
-def infer_fast_path(training, grad_enabled, has_bias, cin, cout, is_cuda, n_out) -> bool:
+def infer_fast_path(training, grad_enabled, has_bias, cin, cout, is_cuda, n_out, kernel_volume=1) -> bool:
     """Whether a convolution forward returns a DeferredConv (inference epilogue, lg_conv_layer_infer): only in eval mode
-    without autograd, on the tensor-core path with one library call per layer and no instrumentation, for a layer
-    without bias whose column blocks are multiples of 32, on a non-empty output.  Everything else runs the forward of
-    training and of eval with gradients unchanged."""
-    return (not training and not grad_enabled and not has_bias and _tc_ok(cin, cout)
+    without autograd, on the tensor-core path (kernel_volume <= TC_MAX_KERNEL_VOLUME; the layers pass theirs) with one
+    library call per layer and no instrumentation, for a layer without bias whose column blocks are multiples of 32, on
+    a non-empty output.  Everything else runs the forward of training and of eval with gradients unchanged."""
+    return (not training and not grad_enabled and not has_bias and _tc_ok(cin, cout, kernel_volume)
             and (cout // ((cout + 255) // 256)) % 32 == 0 and bool(CONFIG["layer_calls"]) and not PROFILE["enabled"]
             and is_cuda and n_out > 0)
 

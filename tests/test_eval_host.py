@@ -179,3 +179,13 @@ def test_eval_bn_coefficients_follow_torch_eval_batch_norm():
     m.train()
     m.eval()
     assert m._eval_stats() is not s2
+
+
+def test_deferred_conv_not_for_more_offsets_than_the_tensor_core_wgrad_takes():
+    """A 5x5x5 layer (125 offsets) runs on the SIMT kernels, so its eval forward is not deferred to the tensor-core
+    inference epilogue either; 3x3x3 and 2x2x2 layers are."""
+    from lidog_b200.me import conv
+    ok = dict(training=False, grad_enabled=False, has_bias=False, cin=32, cout=64, is_cuda=True, n_out=1000)
+    for kv in (1, 8, 27, conv.TC_MAX_KERNEL_VOLUME):
+        assert conv.infer_fast_path(**ok, kernel_volume=kv), kv
+    assert not conv.infer_fast_path(**ok, kernel_volume=125)

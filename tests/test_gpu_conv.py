@@ -106,6 +106,7 @@ TC_CASES = [
     ("down", 1, 2, 32, 32), ("down", 2, 2, 64, 64), ("down", 1, 2, 128, 128),
     ("up", 2, 2, 256, 256), ("up", 2, 2, 256, 128), ("up", 4, 2, 128, 96), ("up", 2, 2, 96, 96),
     ("identity", 1, 1, 32, 64), ("identity", 2, 1, 384, 256), ("identity", 1, 1, 128, 96),
+    ("same", 1, 5, 32, 64),  # kernel volume 125: more offsets than the tensor-core wgrad takes
 ]
 
 
