@@ -320,6 +320,25 @@ int lg_bn_layer_backward(const float* dy, int64_t dy_ld /* row pitch of dy in fl
                          const lgBnBwdBranch* b /* nullable */, float* dres, int32_t fmt, float* scales,
                          const lgPeerCtx* peer /* nullable */, void* stream);
 
+/* ------------------------------------------------------------------ instance norm (+ ReLU, operand cast)
+ *
+ * ME.MinkowskiInstanceNorm, the normalisation of the IBN-Net and RobustNet baselines next to LiDOG (SURVEY.md 2):
+ * instance b = the rows whose batch index coords[r][0] is b (any row order), 1 <= B <= 256 (LG_ERR_UNSUPPORTED above;
+ * rows with a batch index outside [0, B) are left out of the statistics and come out NaN).  Any C >= 1.
+ *   y = act(((x - mean_b) * (var_b + eps)^-1/2) * weight + bias), biased variance, act = ReLU when relu != 0;
+ *   y16 (nullable) = the 16-bit copy (fmt) of y the next tensor-core convolution gathers, equal to lg_cast_rows(y);
+ *   stats double [2][B][C] = mean, invstd (0, 0 for an instance without rows), kept by the caller for the backward.
+ * Features 16-byte aligned when C % 4 == 0.  Scratch: library arena.  Deterministic (fixed-order reductions). */
+int lg_instnorm_forward(const float* x, const int32_t* coords, int64_t n, int32_t C, int32_t B, const float* weight,
+                        const float* bias, float eps, int32_t relu, float* y, void* y16, int32_t fmt, double* stats,
+                        void* stream);
+/* Backward: g = dy * [y > 0] (relu; y is the forward output, else unused and nullable), xhat the normalised x,
+ * dx = invstd * weight * (g - mean_b(g) - xhat * mean_b(g * xhat)), dweight = sum g * xhat, dbias = sum g (all
+ * required outputs, dweight / dbias [C]). */
+int lg_instnorm_backward(const float* dy, const float* x, const float* y, const int32_t* coords, int64_t n, int32_t C,
+                         int32_t B, const float* weight, int32_t relu, const double* stats, float* dx, float* dweight,
+                         float* dbias, void* stream);
+
 /* ------------------------------------------------------------------ SyncBN exchange over peer memory
  *
  * train_lidog.py:228 converts every MinkowskiBatchNorm to SyncBN: 124 latency-bound exchanges of <= 3C doubles per

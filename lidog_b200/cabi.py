@@ -94,6 +94,8 @@ SIGNATURES = {
     "lg_bn_bwd_gscale": (C.c_int, [_vp, _i32, _vp, _vp]),
     "lg_bn_bwd_apply": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _vp,
                                   _vp, _vp, _vp, _vp, _i32, _vp]),
+    "lg_instnorm_forward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _f32, _i32, _vp, _vp, _i32, _vp, _vp]),
+    "lg_instnorm_backward": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "lg_peer_exchange_bytes": (_sz, []),
     "lg_peer_sum": (C.c_int, [_vp, _i32, C.POINTER(C.c_void_p), _i32, _i32, C.c_uint64, _vp, _vp]),
     "lg_dice_forward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _f32, _i32, _vp, _vp, _vp]),
@@ -119,6 +121,7 @@ KERNELS_PER_CALL = {
     "lg_bn_layer_backward": 3, "lg_dice_forward": 2, "lg_dice_backward": 1,
     # + 1 (lg_prep_weights) when the call refreshes the 16-bit weights: counted by the caller
     "lg_conv_layer_infer": 1, "lg_confusion_matrix": 1,
+    "lg_instnorm_forward": 3, "lg_instnorm_backward": 3,
 }
 COUNTS: dict = {}
 _RAW = None

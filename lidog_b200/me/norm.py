@@ -477,13 +477,124 @@ class MinkowskiSyncBatchNorm(MinkowskiBatchNorm):
         return out
 
 
+# ME's eps of MinkowskiInstanceNorm (SURVEY.md Appendix C); the CPU oracle's stand-in normalises with this value too
+INSTANCE_NORM_EPS = 1e-8
+
+
+def _instance_count(t: SparseTensor) -> int:
+    """Instances B of a batch: `coordinate_manager.batch_size` when set, else max batch index + 1 (one host sync,
+    cached on the manager, as lidog/bev.py:sparse2super does)."""
+    cm = t.coordinate_manager
+    B = getattr(cm, "batch_size", None)
+    if B is None:
+        B = int(t.C[:, 0].max().item()) + 1
+        cm.batch_size = B
+    return int(B)
+
+
+class InstanceNormFunction(torch.autograd.Function):
+    """y = act(IN(x) * weight + bias) per instance (csrc/instnorm.cu), ONE library call each way.  The 16-bit copy of
+    y travels in `box`."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, coords, B, relu, box):
+        L = cabi.lib()
+        x = x.contiguous()
+        n, C = x.shape
+        dev = x.device
+        fmt = _fmt16()
+        y = torch.empty_like(x)
+        y16 = torch.empty((n, C), dtype=_dtype16(fmt), device=dev) if fmt is not None else None
+        stats = torch.empty((2, B, C), dtype=torch.float64, device=dev)
+        w, b = weight.detach().reshape(C).contiguous(), bias.detach().reshape(C).contiguous()
+        cabi.check(L.lg_instnorm_forward(x.data_ptr(), coords.data_ptr(), n, C, B, w.data_ptr(), b.data_ptr(),
+                                         INSTANCE_NORM_EPS, 1 if relu else 0, y.data_ptr(), cabi.ptr(y16),
+                                         fmt if fmt is not None else 0, stats.data_ptr(), cabi.stream_of(x)),
+                   "lg_instnorm_forward")
+        box["y16"], box["fmt"] = y16, fmt
+        ctx.save_for_backward(x, y if relu else None, coords, stats, w)
+        ctx.meta = (B, bool(relu), tuple(weight.shape))
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        x, y, coords, stats, w = ctx.saved_tensors
+        B, relu, wshape = ctx.meta
+        dy = dy.contiguous()
+        n, C = x.shape
+        dx = torch.empty_like(x)
+        dwb = torch.empty((2, C), dtype=torch.float32, device=x.device)
+        cabi.check(cabi.lib().lg_instnorm_backward(dy.data_ptr(), x.data_ptr(), cabi.ptr(y), coords.data_ptr(), n, C,
+                                                   B, w.data_ptr(), 1 if relu else 0, stats.data_ptr(), dx.data_ptr(),
+                                                   dwb[0].data_ptr(), dwb[1].data_ptr(), cabi.stream_of(x)),
+                   "lg_instnorm_backward")
+        return dx, dwb[0].view(wshape), dwb[1].view(wshape), None, None, None, None
+
+
+class DeferredIN(SparseTensor):
+    """MinkowskiInstanceNorm output not computed yet: `MinkowskiReLU` evaluates it with the ReLU fused, any other read
+    of `.F` without.  Either way the result carries the 16-bit operand copy for the next convolution."""
+
+    def __init__(self, src: SparseTensor, module):
+        self.coordinate_manager = src.coordinate_manager
+        self._ts = src._ts
+        self._f16_cache = None
+        self._src, self._in = src, module
+        self._value = None
+
+    @property
+    def _F(self):
+        if self._value is None:
+            self._evaluate(False)
+        return self._value
+
+    @_F.setter
+    def _F(self, v):
+        self._value = v
+
+    def _evaluate(self, relu: bool):
+        src, m = self._src, self._in
+        feats = src.F
+        box = {}
+        self._value = InstanceNormFunction.apply(feats, m.weight, m.bias, src.C.contiguous(), _instance_count(src),
+                                                 bool(relu), box)
+        if box.get("y16") is not None:
+            f = self._value
+            self._f16_cache = ((box["fmt"], f._version, f.data_ptr()), box["y16"])
+        self._src = None
+        return self
+
+
+class MinkowskiInstanceNorm(nn.Module):
+    """ME.MinkowskiInstanceNorm: per (instance = batch index, channel) normalisation with the biased variance and
+    eps = INSTANCE_NORM_EPS, then `weight` [1, C] and `bias` [1, C]; no running statistics, so train and eval mode
+    compute the same.  On CUDA float32 features it runs on csrc/instnorm.cu and defers like MinkowskiBatchNorm, so
+    a following MinkowskiReLU joins the same launch."""
+
+    def __init__(self, num_features):
+        super().__init__()
+        self.weight = nn.Parameter(torch.ones(1, num_features))
+        self.bias = nn.Parameter(torch.zeros(1, num_features))
+
+    def forward(self, input: SparseTensor) -> SparseTensor:
+        f = input.F
+        if not (f.is_cuda and f.dtype == torch.float32 and f.dim() == 2):
+            raise RuntimeError("MinkowskiInstanceNorm runs on CUDA float32 features only (csrc/instnorm.cu)")
+        if f.shape[0] == 0:
+            return input._like(torch.empty_like(f))
+        return DeferredIN(input, self)
+
+    def __repr__(self):
+        return f"{self.__class__.__name__}({self.weight.shape[1]})"
+
+
 class MinkowskiReLU(nn.Module):
     def __init__(self, inplace=False):
         super().__init__()
         self.inplace = inplace
 
     def forward(self, input: SparseTensor) -> SparseTensor:
-        if isinstance(input, DeferredBN) and input._value is None:
+        if isinstance(input, (DeferredBN, DeferredIN)) and input._value is None:
             return input._evaluate(True)
         if isinstance(input, DeferredConv) and input._value is None and input._bn_stats is not None:
             return input._launch(True)

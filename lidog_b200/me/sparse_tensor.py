@@ -15,6 +15,27 @@ from .. import cabi
 from .coords import CoordinateManager
 
 
+class CoordinateMapKey:
+    """Names the coordinate map of a tensor within its manager, as ME's key does: here the tensor stride is all there
+    is to it.  `SparseTensor(features=..., coordinate_map_key=t.coordinate_map_key,
+    coordinate_manager=t.coordinate_manager)` puts new features on t's coordinates (IBN-style channel splits)."""
+
+    def __init__(self, tensor_stride):
+        self._ts = int(tensor_stride[0] if isinstance(tensor_stride, (list, tuple)) else tensor_stride)
+
+    def get_tensor_stride(self):
+        return [self._ts] * 3
+
+    def __eq__(self, other):
+        return isinstance(other, CoordinateMapKey) and other._ts == self._ts
+
+    def __hash__(self):
+        return hash(("CoordinateMapKey", self._ts))
+
+    def __repr__(self):
+        return f"CoordinateMapKey(tensor_stride={self.get_tensor_stride()})"
+
+
 class SparseTensor:
     _stat_partials = None  # (per-tile column statistics written by the producing convolution's epilogue, F version)
 
@@ -26,6 +47,8 @@ class SparseTensor:
             tensor_stride = tensor_stride[0]
         if device is not None:
             features = features.to(device)
+        if coordinate_map_key is not None and coordinate_manager is not None:
+            tensor_stride = coordinate_map_key._ts
         if coordinate_manager is None:
             if coordinates is None:
                 raise ValueError("either coordinates or a coordinate_manager is required")
@@ -58,6 +81,10 @@ class SparseTensor:
     @property
     def tensor_stride(self):
         return [self._ts] * 3
+
+    @property
+    def coordinate_map_key(self):
+        return CoordinateMapKey(self._ts)
 
     @property
     def device(self):
