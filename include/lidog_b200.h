@@ -374,21 +374,26 @@ int lg_confusion_matrix(const float* logits, int64_t n, int32_t C, const int64_t
 
 /* ------------------------------------------------------------------ BEV projection */
 
-size_t lg_bev_workspace(int64_t n, int32_t C, int32_t batch_size, int32_t H, int32_t W);
+/* Bytes of the workspace that lg_bev_forward fills and lg_bev_backward reads, for the same arguments.  It holds the
+ * pixel map, the row-occupancy words and the winning cell of every pooling window (one byte per output element:
+ * ~340 MB at batch 8, C = 96, 2000 x 2000 -> 666 x 666). */
+size_t lg_bev_workspace(int64_t n, int32_t C, int32_t batch_size, int32_t H, int32_t W, int32_t pk, int32_t ps,
+                        int32_t pp);
 
 /* Fused point-to-BEV projection: pixel scatter + raw (H,W,C)->(C,H,W) re-view + MaxPool2d(pk,ps,pp),
  * never materialising the dense tensor.  Replaces MinkUNetBaseBEV.sparse2super + filter_bounds
  * (utils/models/minkunet_bev.py:158-230).  out: float [batch, C, h, w], h = (H + 2pp - pk)/ps + 1, stored
  * NCHW (layout 0) or NHWC / channels_last (layout 1: the same logical tensor, the memory order cuDNN's
  * tensor-op convolutions of the dense 2D head consume without staging copies).
- * workspace keeps the pixel map and the row-occupancy words for lg_bev_backward. */
+ * workspace keeps the pixel map, the row-occupancy words and each window's winning cell for lg_bev_backward. */
 int lg_bev_forward(const int32_t* coords4, const float* feats, int64_t n, int32_t C, int32_t batch_size, float bound,
                    float voxel_size, int32_t H, int32_t W, int32_t pk, int32_t ps, int32_t pp, int32_t policy,
                    int32_t layout, float* out, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Backward of the above (autograd of index_put_ + max_pool2d at minkunet_bev.py:217-221).
- * grad_feats [n, C] is fully written.  Atomic-free and bit-reproducible: every occupied cell sums the <= 4 windows it
- * won in ascending (i, j) order (the order of torch's CPU max_pool2d backward). */
+ * grad_feats [n, C] is fully written (rows outside the image get 0).  Atomic-free and bit-reproducible: every occupied
+ * cell sums the <= 4 windows it won in ascending (i, j) order (the order of torch's CPU max_pool2d backward).
+ * workspace: as the forward left it. */
 int lg_bev_backward(const int32_t* coords4, const float* feats, int64_t n, int32_t C, int32_t batch_size,
                     int32_t H, int32_t W, int32_t pk, int32_t ps, int32_t pp, int32_t policy, int32_t layout,
                     const float* grad_out, float* grad_feats, const void* workspace, size_t workspace_bytes,

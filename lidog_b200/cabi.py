@@ -100,7 +100,7 @@ SIGNATURES = {
     "lg_peer_sum": (C.c_int, [_vp, _i32, C.POINTER(C.c_void_p), _i32, _i32, C.c_uint64, _vp, _vp]),
     "lg_dice_forward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _f32, _i32, _vp, _vp, _vp]),
     "lg_dice_backward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _f32, _i32, _vp, _vp, _vp, _vp]),
-    "lg_bev_workspace": (_sz, [_i64, _i32, _i32, _i32, _i32]),
+    "lg_bev_workspace": (_sz, [_i64, _i32, _i32, _i32, _i32, _i32, _i32, _i32]),
     "lg_bev_forward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _f32, _f32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp,
                                  _vp, _sz, _vp]),
     "lg_bev_backward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp,
@@ -115,7 +115,7 @@ KERNELS_PER_CALL = {
     "lg_quantize_points": 1, "lg_quantize_points_f64": 1, "lg_coords_unique": 7, "lg_kernel_map": 1, "lg_kernel_map_sorted": 7, "lg_kernel_map_pairs": 3,
     "lg_kernel_map_up2": 9, "lg_conv_gemm_simt": 1, "lg_conv_wgrad_simt": 2, "lg_cast_rows": 1,
     "lg_absmax_scale": 2, "lg_prep_weights": 1, "lg_conv_gemm_tc": 1, "lg_conv_wgrad_tc": 2,
-    "lg_bev_forward": 2, "lg_bev_backward": 3,
+    "lg_bev_forward": 2, "lg_bev_backward": 1,
     "lg_bn_stats": 2, "lg_bn_finalize": 1, "lg_bn_apply": 1, "lg_bn_bwd_stats": 2, "lg_bn_bwd_finalize": 1,
     "lg_bn_bwd_gscale": 1, "lg_bn_bwd_apply": 1, "lg_peer_sum": 1,
     "lg_bn_layer_backward": 3, "lg_dice_forward": 2, "lg_dice_backward": 1,

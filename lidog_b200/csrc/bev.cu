@@ -15,9 +15,11 @@
 // the lines pool zeros only.  Now an occupancy word per scrambled row (`rowbits`, built by one scatter over the
 // voxels: bit jt = "this row holds a voxel inside tile column block jt") answers the emptiness question with 32
 // coalesced loads per tile, only occupied rows touch the pixel map, only non-empty lines are scanned, and tiles move
-// as float4.  The backward is atomic-free: a tile also evaluates the windows one row above / one column left of it
-// (halo) and every occupied cell adds up the <= 4 windows it won in ascending (i, j) order -- the order of torch's CPU
-// max_pool2d backward, so the gradient is reproduced bit for bit and is run-to-run deterministic.
+// as float4.  While it scans, the forward records the winning cell of every window that can hold a voxel in a
+// one-byte-per-window table (`argpos`).  The backward is one pass over the voxel rows, a warp per row and a lane per
+// channel: each (row, channel) cell adds up the <= 2 x 2 windows the table says it won, in ascending (i, j) order --
+// the order of torch's CPU max_pool2d backward, so the gradient is reproduced bit for bit -- and every element of the
+// gradient is written by exactly one thread: no atomics, no memset, run-to-run deterministic.
 #include "common.cuh"
 
 namespace lg {
@@ -27,10 +29,12 @@ struct BevWorkspace {
   int* next;        // [n]      chain of rows sharing a pixel (LG_BEV_MAX)
   int* pixmap;      // [B*H*W]  winner row (LAST) / chain head (MAX) / -1
   uint32_t* rowbits;  // [B*C*H]  bit jt: scrambled row (c', h') holds a voxel inside tile column block jt
+  unsigned char* argpos;  // [B*C*h_out*w_out] winning cell of a window ((h - h0) * pk + w - w0; 255 = an empty cell);
+                          // written only for the (c', i) lines that can hold a voxel, which every voxel's window is on
   size_t total;
 };
 
-static BevWorkspace carve_bev(void* base, int64_t n, int64_t pixels, int64_t rows) {
+static BevWorkspace carve_bev(void* base, int64_t n, int64_t pixels, int64_t rows, int64_t windows) {
   BevWorkspace w;
   size_t off = 0;
   auto take = [&](size_t bytes) {
@@ -42,6 +46,7 @@ static BevWorkspace carve_bev(void* base, int64_t n, int64_t pixels, int64_t row
   w.next = (int*)take(sizeof(int) * (size_t)(n > 0 ? n : 1));
   w.pixmap = (int*)take(sizeof(int) * (size_t)pixels);
   w.rowbits = (uint32_t*)take(sizeof(uint32_t) * (size_t)rows);
+  w.argpos = (unsigned char*)take((size_t)windows);
   w.total = off;
   return w;
 }
@@ -141,7 +146,6 @@ constexpr int kCG = 32;   // scrambled channels per CTA
 constexpr int kIB = 8;    // output rows per CTA
 constexpr int kJC = 32;   // output columns per CTA
 constexpr int kPitch = kCG + 4;  // floats per staged (i, j) cell group: float4-aligned, conflict-free 128-bit reads
-constexpr int kIBh = kIB + 1;  // backward: window rows including the halo row above
 
 struct TileGeom {
   int b, c0, i0, j0;  // sample, first scrambled channel, first window row / column handled
@@ -178,20 +182,17 @@ __device__ __forceinline__ TileGeom tile_geom(int C, int H, int W, int h_out, in
 }
 
 struct TileSmem {
-  float* out;         // staged results (forward) / gradients (backward): [rows][cols][kPitch]
+  float* out;         // staged results: [rows][cols][kPitch]
   int* heads;         // [pairs][max_pix] pixel -> row head (or -1); valid for rows whose rowmask bit is set
   int* plo;           // [pairs] first pixel of the run
   uint32_t* rowmask;  // [kCG] bit (h - h_lo): scrambled row h of channel c' holds a voxel
   unsigned short* lines;  // non-empty (c', i) lines of the tile: (cl << 8) | il; *n_lines = their count
   int* n_lines;
-  int* list;          // backward: occupied (pair, pixel) entries of the tile; list[-1] = their count
-  unsigned char* arg; // backward: [kCG][kIBh][kJC] winning cell of every window (position in the window, 255 = none)
 };
 
 // Phase 1.  Returns false (uniformly) when no pixel of the tile is occupied.  One coalesced rowbits load per
 // scrambled channel (lane = scrambled row, nrows <= 32 host-checked); only rows whose occupancy bit is set go to the
-// pixel map.  WITH_LIST also records the occupied (pair, pixel) entries for the backward's owner-computes pass.
-template <bool WITH_LIST>
+// pixel map.
 __device__ __forceinline__ bool tile_lookup(const TileGeom& g, const TileSmem& t, int C, int H, int W, int max_pix,
                                             const int* __restrict__ pixmap, const uint32_t* __restrict__ rowbits) {
   const int nrows = g.h_hi - g.h_lo;
@@ -210,10 +211,7 @@ __device__ __forceinline__ bool tile_lookup(const TileGeom& g, const TileSmem& t
       for (int d = 0; d < max_pix; ++d) {
         const int head = (p_lo + d <= p_hi) ? __ldg(pm + p_lo + d) : -1;
         t.heads[q * max_pix + d] = head;
-        if (head >= 0) {
-          row_any = 1;
-          if (WITH_LIST) t.list[atomicAdd(t.list - 1, 1)] = q * max_pix + d;
-        }
+        if (head >= 0) row_any = 1;
       }
     }
     const uint32_t bits = __ballot_sync(0xffffffffu, row_any);
@@ -224,26 +222,23 @@ __device__ __forceinline__ bool tile_lookup(const TileGeom& g, const TileSmem& t
 }
 
 // Scan of one window in the reference's order (rows, then columns; strict > keeps the first maximum).
-// Returns the pooled value.  WANT_ARG: *arg_row = voxel row of the winning cell (-1 when an empty cell wins;
-// MAX policy: -2 - chain head, resolved lazily), *arg_ch its channel, *arg_pos its position (h - h0) * pk + (w - w0)
-// inside the window.
-template <bool WANT_ARG>
+// Returns the pooled value; *pos = position (h - h0) * pk + (w - w0) of the winning cell inside the window, 255 when
+// an empty cell (a zero) wins.
 __device__ __forceinline__ float window_scan(const TileGeom& g, const TileSmem& t, int cl, int i, int j, int C, int H,
                                              int W, int pk, int ps, int pp, int max_pix, int policy,
-                                             const float* __restrict__ feats, const int* __restrict__ next,
-                                             int* arg_row, int* arg_ch, int* arg_pos) {
+                                             const float* __restrict__ feats, const int* __restrict__ next, int* pos) {
   const int nrows = g.h_hi - g.h_lo;
   const int h0 = i * ps - pp, w0 = j * ps - pp;
   const int ha = max(h0, 0), hb = min(h0 + pk, H), wa = max(w0, 0), wb = min(w0 + pk, W);
   const uint32_t rbits = (t.rowmask[cl] >> (ha - g.h_lo)) & ((1u << (hb - ha)) - 1u);
-  if (WANT_ARG) *arg_row = -1;
+  *pos = 255;
   if (!rbits) return 0.f;  // every cell is an empty zero; the first one wins
   float best = -INFINITY;
   for (int h = ha; h < hb; ++h) {
     if (!((rbits >> (h - ha)) & 1u)) {  // an all-empty row: zeros
       if (0.f > best) {
         best = 0.f;
-        if (WANT_ARG) *arg_row = -1;
+        *pos = 255;
       }
       continue;
     }
@@ -261,18 +256,14 @@ __device__ __forceinline__ float window_scan(const TileGeom& g, const TileSmem& 
       if (head < 0) {  // a run of empty zeros; only its first cell can take the lead
         if (0.f > best) {
           best = 0.f;
-          if (WANT_ARG) *arg_row = -1;
+          *pos = 255;
         }
       } else {
         for (int k = 0; k < span; ++k) {
           const float v = cell_value(head, ch + k, C, policy, feats, next);
           if (v > best) {
             best = v;
-            if (WANT_ARG) {
-              *arg_row = (policy == LG_BEV_LAST) ? head : -2 - head;
-              *arg_ch = ch + k;
-              *arg_pos = (h - h0) * pk + (w + k - w0);
-            }
+            *pos = (h - h0) * pk + (w + k - w0);
           }
         }
       }
@@ -350,20 +341,17 @@ __device__ __forceinline__ uint32_t line_row_bits(const TileGeom& g, const TileS
 // channel, so the non-empty lines of a tile belong to a few c' -- with one warp per c' most warps idled at the barrier.
 // `*t.n_lines` must be zero on entry; every thread of the CTA calls this.
 __device__ __forceinline__ void collect_lines(const TileGeom& g, const TileSmem& t, int H, int pk, int ps, int pp) {
-  {
-    const int cl = threadIdx.x >> 3, il = threadIdx.x & 7;
-    if (cl < g.ncg && il < g.nib && line_row_bits(g, t, cl, g.i0 + il, H, pk, ps, pp))
-      t.lines[atomicAdd(t.n_lines, 1)] = (unsigned short)((cl << 8) | il);
-  }
-  if (g.nib > 8 && threadIdx.x < g.ncg && line_row_bits(g, t, threadIdx.x, g.i0 + 8, H, pk, ps, pp))  // the halo's 9th row
-    t.lines[atomicAdd(t.n_lines, 1)] = (unsigned short)((threadIdx.x << 8) | 8);
+  const int cl = threadIdx.x >> 3, il = threadIdx.x & 7;
+  if (cl < g.ncg && il < g.nib && line_row_bits(g, t, cl, g.i0 + il, H, pk, ps, pp))
+    t.lines[atomicAdd(t.n_lines, 1)] = (unsigned short)((cl << 8) | il);
   __syncthreads();
 }
 
 __global__ void __launch_bounds__(256)
     k_bev_pool_fwd(const float* __restrict__ feats, const int* __restrict__ next, const int* __restrict__ pixmap,
                    const uint32_t* __restrict__ rowbits, int C, int H, int W, int h_out, int w_out, int pk, int ps,
-                   int pp, int policy, int layout, int max_pix, int pairs_cap, float* __restrict__ out) {
+                   int pp, int policy, int layout, int max_pix, int pairs_cap, float* __restrict__ out,
+                   unsigned char* __restrict__ argpos) {
   extern __shared__ __align__(16) unsigned char s_dyn[];
   TileSmem t;
   t.out = reinterpret_cast<float*>(s_dyn);
@@ -372,8 +360,6 @@ __global__ void __launch_bounds__(256)
   t.rowmask = reinterpret_cast<uint32_t*>(t.plo + pairs_cap);
   t.n_lines = reinterpret_cast<int*>(t.rowmask + kCG);
   t.lines = reinterpret_cast<unsigned short*>(t.n_lines + 1);
-  t.list = nullptr;
-  t.arg = nullptr;
   const TileGeom g = tile_geom(C, H, W, h_out, w_out, pk, ps, pp);
   {  // zero the staged tile: most lines pool zeros only and are never touched again
     float4* o4 = reinterpret_cast<float4*>(t.out);
@@ -381,17 +367,20 @@ __global__ void __launch_bounds__(256)
     for (int u = threadIdx.x; u < kIB * kJC * kPitch / 4; u += blockDim.x) o4[u] = z;
     if (threadIdx.x == 0) *t.n_lines = 0;
   }
-  if (tile_lookup<false>(g, t, C, H, W, max_pix, pixmap, rowbits)) {
+  if (tile_lookup(g, t, C, H, W, max_pix, pixmap, rowbits)) {
     collect_lines(g, t, H, pk, ps, pp);
     // a warp takes one non-empty (c', i) line at a time, lane = column: the 32 windows of a line share their
-    // scrambled rows and neighbouring lanes read neighbouring cells
+    // scrambled rows and neighbouring lanes read neighbouring cells (and write neighbouring bytes of argpos)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int n_lines = *t.n_lines;
     for (int e = warp; e < n_lines; e += 8) {
       const int cl = t.lines[e] >> 8, il = t.lines[e] & 255;
-      if (lane < g.njc)
-        t.out[(il * kJC + lane) * kPitch + cl] = window_scan<false>(g, t, cl, g.i0 + il, g.j0 + lane, C, H, W, pk, ps, pp,
-                                                                    max_pix, policy, feats, next, nullptr, nullptr, nullptr);
+      if (lane < g.njc) {
+        int pos;
+        t.out[(il * kJC + lane) * kPitch + cl] = window_scan(g, t, cl, g.i0 + il, g.j0 + lane, C, H, W, pk, ps, pp,
+                                                             max_pix, policy, feats, next, &pos);
+        argpos[(((int64_t)g.b * C + g.c0 + cl) * h_out + g.i0 + il) * w_out + g.j0 + lane] = (unsigned char)pos;
+      }
     }
     __syncthreads();
   }
@@ -399,134 +388,73 @@ __global__ void __launch_bounds__(256)
 }
 
 // Backward.  The gradient of a window goes to its first arg-max in scan order (max_pool2d backward) if that cell
-// holds a voxel; a cell sits in <= 2 x 2 windows (host-checked: pk <= 2 ps).  Owner computes: the tile that owns the
-// LAST window (largest i, j) containing a cell sums the cell's windows in ascending (i, j) order -- for that it also
-// scans the windows one row above and one column left of its own (halo).  Every gradient element is written by
-// exactly one thread with a fixed summation order: no atomics, bit-reproducible, and equal to torch's CPU backward.
-// A tile owns kIB x kJB = 8 x 31 windows, so that owned + halo columns fill exactly one warp (a 33rd column made every
-// line cost two passes); the window gradients are read from global memory only for the windows a cell actually won
-// (no staged copy of the gradient tile: 43 KB of shared memory and 10 % of the instructions in the first version).
-constexpr int kJB = kJC - 1;  // owned window columns of a backward tile
-
-__device__ __forceinline__ float grad_at(const float* __restrict__ grad_out, int layout, int b, int c, int i, int j, int C,
-                                         int h_out, int w_out) {
-  return __ldg(grad_out + (layout ? (((int64_t)b * h_out + i) * w_out + j) * C + c
-                                  : (((int64_t)b * C + c) * h_out + i) * w_out + j));
-}
-
+// holds a voxel; the forward left the cell's position in `argpos`.  A warp owns one voxel row, lane = channel, so the
+// row's writes are coalesced.  The row's cell (c', h, w) sits in <= 2 x 2 windows (host-checked: pk <= 2 ps) and adds
+// up those whose table entry names it in ascending (i, j) order -- the order of torch's CPU max_pool2d backward, so
+// the gradient is bit-equal to it.  LAST: every row of the pixel computes the same sum (index_put_ backward hands the
+// pixel's gradient to each row that wrote it); MAX: only the chain's first row attaining the cell's max receives it.
+// Every element of grad_feats is written exactly once, rows outside the image with 0: no memset, no atomics.
 __global__ void __launch_bounds__(256)
-    k_bev_pool_bwd(const float* __restrict__ feats, const int* __restrict__ next, const int* __restrict__ pixmap,
-                   const uint32_t* __restrict__ rowbits, int C, int H, int W, int h_out, int w_out, int pk, int ps,
-                   int pp, int policy, int layout, int max_pix, int pairs_cap, const float* __restrict__ grad_out,
-                   float* __restrict__ grad_feats) {
-  extern __shared__ __align__(16) unsigned char s_dyn[];
-  TileSmem t;
-  t.out = nullptr;
-  t.heads = reinterpret_cast<int*>(s_dyn);
-  t.plo = t.heads + pairs_cap * max_pix;
-  t.rowmask = reinterpret_cast<uint32_t*>(t.plo + pairs_cap);
-  t.n_lines = reinterpret_cast<int*>(t.rowmask + kCG);
-  t.list = t.n_lines + 2;  // list[-1] = number of entries
-  t.arg = reinterpret_cast<unsigned char*>(t.list + pairs_cap * max_pix);
-  t.lines = reinterpret_cast<unsigned short*>(t.arg + kCG * kIBh * kJC);
-  // owned windows
-  TileGeom own;
-  {
-    const int n_jb = (w_out + kJB - 1) / kJB, n_ib = (h_out + kIB - 1) / kIB, n_cg = (C + kCG - 1) / kCG;
-    int idx = blockIdx.x;
-    own.jt = idx % n_jb;
-    own.j0 = own.jt * kJB;
-    idx /= n_jb;
-    own.i0 = (idx % n_ib) * kIB;
-    idx /= n_ib;
-    own.c0 = (idx % n_cg) * kCG;
-    own.b = idx / n_cg;
-    own.ncg = min(kCG, C - own.c0);
-    own.nib = min(kIB, h_out - own.i0);
-    own.njc = min(kJB, w_out - own.j0);
+    k_bev_pool_bwd(const float* __restrict__ feats, const int* __restrict__ pix_of_row, const int* __restrict__ next,
+                   const int* __restrict__ pixmap, const unsigned char* __restrict__ argpos, int64_t n, int C, int H,
+                   int W, int h_out, int w_out, int pk, int ps, int pp, int policy, int layout,
+                   const float* __restrict__ grad_out, float* __restrict__ grad_feats) {
+  const int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (r >= n) return;
+  const int lane = threadIdx.x & 31;
+  float* gf = grad_feats + r * C;
+  const int pix = __ldg(pix_of_row + r);
+  if (pix < 0) {
+    for (int ch = lane; ch < C; ch += 32) gf[ch] = 0.f;
+    return;
   }
-  TileGeom g = own;  // windows handled = owned + halo
-  g.i0 = max(own.i0 - 1, 0);
-  g.j0 = max(own.j0 - 1, 0);
-  g.nib = own.i0 + own.nib - g.i0;
-  g.njc = own.j0 + own.njc - g.j0;
-  cell_region(g, H, W, pk, ps, pp);
-  {  // occupancy bits of the forward's column blocks (kJC windows wide) that overlap this tile's cell columns
-    const int bw = kJC * ps, cover = (kJC - 1) * ps + pk, n_jc = (w_out + kJC - 1) / kJC;
-    int lo = g.w_lo + pp - cover + 1;
-    lo = lo <= 0 ? 0 : (lo + bw - 1) / bw;
-    const int hi = min(n_jc - 1, (g.w_hi - 1 + pp) / bw);
-    g.jbits = (hi - lo == 31) ? 0xffffffffu : (((1u << (hi - lo + 1)) - 1u) << lo);
-  }
-  if (threadIdx.x == 0) t.list[-1] = 0, *t.n_lines = 0;
-  __syncthreads();
-  if (!tile_lookup<true>(g, t, C, H, W, max_pix, pixmap, rowbits)) return;
-  static_assert((kCG * kIBh * kJC) % 4 == 0, "winning-cell table is filled word-wise");
-  for (int u = threadIdx.x; u < kCG * kIBh * kJC / 4; u += blockDim.x) reinterpret_cast<uint32_t*>(t.arg)[u] = 0xffffffffu;
-  collect_lines(g, t, H, pk, ps, pp);  // (ends with a barrier: the table above is complete too)
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  // phase A: winning cell of every window of the non-empty lines (shared by all warps); lane = window column
-  const int n_lines = *t.n_lines;
-  for (int e = warp; e < n_lines; e += 8) {
-    const int cl = t.lines[e] >> 8, il = t.lines[e] & 255;
-    if (lane < g.njc) {
-      int row = -1, ch = 0, pos = 255;
-      window_scan<true>(g, t, cl, g.i0 + il, g.j0 + lane, C, H, W, pk, ps, pp, max_pix, policy, feats, next, &row, &ch,
-                        &pos);
-      if (row != -1) t.arg[(cl * kIBh + il) * kJC + lane] = (unsigned char)pos;
-    }
-  }
-  __syncthreads();
-  // phase B: every occupied cell this tile owns sums the windows it won
-  const int nrows = g.h_hi - g.h_lo;
-  const int n_list = t.list[-1];
-  for (int e = warp; e < n_list; e += 8) {
-    const int qd = t.list[e];
-    const int q = qd / max_pix, d = qd - q * max_pix;
-    const int cl = q / nrows, h = g.h_lo + (q - cl * nrows);
-    const int head = t.heads[qd];
-    const int m_row = ((g.c0 + cl) * H + h) * W;
-    const int p = t.plo[q] + d;
-    const int m_a = max(p * C, m_row + g.w_lo), m_b = min(p * C + C, m_row + g.w_hi);
-    const int i_hi = min((h + pp) / ps, h_out - 1);
-    if (h > i_hi * ps - pp + pk - 1) continue;  // below the last window: the cell is pooled by nobody
-    if (i_hi < own.i0 || i_hi >= own.i0 + own.nib) continue;  // another tile owns this row of cells
-    const int i_lo = max((h + pp - pk + ps) / ps, 0);
-    for (int m = m_a + lane; m < m_b; m += 32) {
-      const int w = m - m_row, ch = m - p * C;
-      const int j_hi = min((w + pp) / ps, w_out - 1);
-      if (w > j_hi * ps - pp + pk - 1) continue;
-      if (j_hi < own.j0 || j_hi >= own.j0 + own.njc) continue;
-      const int j_lo = max((w + pp - pk + ps) / ps, 0);
-      float sum = 0.f;
-      bool hit = false;
-      for (int i = i_lo; i <= i_hi; ++i)
-        for (int j = j_lo; j <= j_hi; ++j) {
-          const int pos = (h - (i * ps - pp)) * pk + (w - (j * ps - pp));
-          if (t.arg[(cl * kIBh + (i - g.i0)) * kJC + (j - g.j0)] == pos) {
-            sum += grad_at(grad_out, layout, g.b, g.c0 + cl, i, j, C, h_out, w_out);
-            hit = true;
+  const int hw = H * W, b = pix / hw;
+  const int head = policy == LG_BEV_MAX ? __ldg(pixmap + pix) : -1;
+  const int m0 = (pix - b * hw) * C;  // flat index of the row's first cell in the sample's dense buffer
+  const int64_t sample = (int64_t)b * C * h_out * w_out;  // C * h_out * w_out < 2^31 (host-checked)
+  const unsigned char* tab = argpos + sample;
+  const float* go = grad_out + sample;
+  // kU channels per lane at a time, unrolled, so that their table reads and then their gradient reads are in flight
+  // together: one channel at a time left a chain of dependent loads per channel and the pass latency-bound (0.77 ms
+  // at the bench shape).  3 takes the bench's 96 channels in one pass (0.64 ms); 4 needs 68 registers, keeps fewer
+  // warps resident and measured 0.80 ms (profiles/r05_bev_bench.jsonl).
+  constexpr int kU = 3;
+  for (int base = lane; base < C; base += 32 * kU) {
+    bool hit[kU][4];
+    int off[kU][4];
+#pragma unroll
+    for (int k = 0; k < kU; ++k) {
+      const int ch = base + 32 * k;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) hit[k][q] = false, off[k][q] = 0;
+      if (ch < C && (policy == LG_BEV_LAST || cell_argrow(head, ch, C, policy, feats, next) == (int)r)) {
+        // scrambled cell (c', h, w): the (H, W, C) buffer re-viewed as (C, H, W); m < C * H * W < 2^31 (host-checked)
+        const int m = m0 + ch, c = m / hw, h = (m - c * hw) / W, w = m - c * hw - h * W;
+        // window rows containing h: qi - 1 (h at row offset ri + ps) and qi (offset ri), where it lies inside them
+        const int qi = (unsigned)(h + pp) / (unsigned)ps, ri = h + pp - qi * ps;
+        const int qj = (unsigned)(w + pp) / (unsigned)ps, rj = w + pp - qj * ps;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {  // ascending (i, j)
+          const int di = 1 - (q >> 1), dj = 1 - (q & 1);
+          const int i = qi - di, j = qj - dj, oh = ri + di * ps, ow = rj + dj * ps;
+          if (i >= 0 && i < h_out && oh < pk && j >= 0 && j < w_out && ow < pk) {
+            const int t = (c * h_out + i) * w_out + j;
+            hit[k][q] = __ldg(tab + t) == oh * pk + ow;
+            off[k][q] = layout ? (i * w_out + j) * C + c : t;
           }
         }
-      if (hit) {
-        const int row = cell_argrow(head, ch, C, policy, feats, next);
-        grad_feats[(int64_t)row * C + ch] = sum;
       }
     }
+#pragma unroll
+    for (int k = 0; k < kU; ++k) {
+      const int ch = base + 32 * k;
+      float sum = 0.f;
+#pragma unroll
+      for (int q = 0; q < 4; ++q)
+        if (hit[k][q]) sum += __ldg(go + off[k][q]);
+      if (ch < C) gf[ch] = sum;
+    }
   }
-}
-
-// LG_BEV_LAST: every row that wrote the pixel receives the pixel's gradient (index_put_ backward)
-__global__ void __launch_bounds__(256)
-    k_bev_dup_grad(const int* __restrict__ pix_of_row, const int* __restrict__ pixmap, int64_t n, int C,
-                   float* __restrict__ grad_feats) {
-  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= n * C) return;
-  const int64_t r = e / C;
-  const int pix = pix_of_row[r];
-  if (pix < 0) return;
-  const int w = pixmap[pix];
-  if (w != (int)r) grad_feats[e] = grad_feats[(int64_t)w * C + (e - r * C)];
 }
 
 }  // namespace lg
@@ -541,14 +469,14 @@ static size_t bev_smem_fwd(int C, int pk, int ps) {  // staged tile + heads + fi
   return sizeof(float) * kIB * kJC * kPitch + sizeof(int) * pairs * (bev_max_pix(C, pk, ps, kJC) + 1) + sizeof(int) * kCG +
          sizeof(int) + 2 * kCG * kIB + 16;
 }
-static size_t bev_smem_bwd(int C, int pk, int ps) {  // heads + first pixels + masks + occupied-entry list + winning cells
-  const size_t pairs = bev_pairs_cap(C, pk, ps, kIBh);
-  const size_t mp = bev_max_pix(C, pk, ps, kJC);
-  return sizeof(int) * pairs * (mp + 1) + sizeof(int) * kCG + sizeof(int) * (pairs * mp + 2) + (size_t)kCG * kIBh * kJC +
-         2 * kCG * kIBh + 32;
+static int64_t bev_tiles(int B, int C, int h_out, int w_out) {
+  return (int64_t)B * ceil_div(C, kCG) * ceil_div(h_out, kIB) * ceil_div(w_out, kJC);
 }
-static int64_t bev_tiles(int B, int C, int h_out, int w_out, int cols = kJC) {
-  return (int64_t)B * ceil_div(C, kCG) * ceil_div(h_out, kIB) * ceil_div(w_out, cols);
+// pooling windows of the output (entries of the argpos table); 0 for parameters bev_check rejects
+static int64_t bev_windows(int B, int C, int H, int W, int pk, int ps, int pp) {
+  if (B < 1 || C < 1 || ps < 1) return 0;
+  const int64_t h_out = (H + 2 * pp - pk) / ps + 1, w_out = (W + 2 * pp - pk) / ps + 1;
+  return h_out > 0 && w_out > 0 ? (int64_t)B * C * h_out * w_out : 0;
 }
 
 static int bev_check(int64_t n, int C, int B, int H, int W, int pk, int ps, int pp, int policy, const char* who) {
@@ -559,14 +487,17 @@ static int bev_check(int64_t n, int C, int B, int H, int W, int pk, int ps, int 
   LG_CHECK_ARG(kIB * ps + pk <= 32, "%s: pool stride/kernel too large for the row mask", who);
   LG_CHECK_ARG(pk <= 2 * ps && pk * pk < 255, "%s: a cell may sit in at most 2 x 2 windows (pk <= 2 ps)", who);
   LG_CHECK_ARG((int64_t)C * H * W < ((int64_t)1 << 31), "%s: C*H*W exceeds int32", who);
-  const int w_out = (W + 2 * pp - pk) / ps + 1;
+  const int h_out = (H + 2 * pp - pk) / ps + 1, w_out = (W + 2 * pp - pk) / ps + 1;
+  LG_CHECK_ARG((int64_t)C * h_out * w_out < ((int64_t)1 << 31), "%s: C*h_out*w_out exceeds int32", who);
   LG_CHECK_ARG(ceil_div(w_out, kJC) <= 32, "%s: more than 32 tile column blocks (W too large for the occupancy word)", who);
-  LG_CHECK_ARG(bev_smem_bwd(C, pk, ps) <= 200 * 1024, "%s: C=%d too small for pool stride %d (shared memory)", who, C, ps);
+  LG_CHECK_ARG(bev_smem_fwd(C, pk, ps) <= 200 * 1024, "%s: C=%d too small for pool stride %d (shared memory)", who, C, ps);
   return LG_OK;
 }
 
-extern "C" size_t lg_bev_workspace(int64_t n, int32_t C, int32_t batch_size, int32_t H, int32_t W) {
-  return carve_bev(nullptr, n, (int64_t)batch_size * H * W, (int64_t)batch_size * C * H).total;
+extern "C" size_t lg_bev_workspace(int64_t n, int32_t C, int32_t batch_size, int32_t H, int32_t W, int32_t pk,
+                                   int32_t ps, int32_t pp) {
+  const int64_t windows = bev_windows(batch_size, C, H, W, pk, ps, pp);
+  return carve_bev(nullptr, n, (int64_t)batch_size * H * W, (int64_t)batch_size * C * H, windows).total;
 }
 
 extern "C" int lg_bev_forward(const int32_t* coords4, const float* feats, int64_t n, int32_t C, int32_t batch_size,
@@ -577,7 +508,7 @@ extern "C" int lg_bev_forward(const int32_t* coords4, const float* feats, int64_
   int rc = bev_check(n, C, batch_size, H, W, pk, ps, pp, policy, "lg_bev_forward");
   if (rc) return rc;
   const int64_t pixels = (int64_t)batch_size * H * W, rows = (int64_t)batch_size * C * H;
-  BevWorkspace w = carve_bev(workspace, n, pixels, rows);
+  BevWorkspace w = carve_bev(workspace, n, pixels, rows, bev_windows(batch_size, C, H, W, pk, ps, pp));
   LG_CHECK_ARG(workspace && workspace_bytes >= w.total, "lg_bev_forward: workspace too small");
   LG_CHECK_ARG(out && (n == 0 || (coords4 && feats)), "lg_bev_forward: null pointer");
   LG_CHECK_ARG(layout == 0 || layout == 1, "lg_bev_forward: layout must be 0 (NCHW) or 1 (NHWC)");
@@ -601,7 +532,7 @@ extern "C" int lg_bev_forward(const int32_t* coords4, const float* feats, int64_
   LG_CUDA_OK(cudaFuncSetAttribute(k_bev_pool_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k_bev_pool_fwd<<<(unsigned)blocks, 256, smem, stream>>>(feats, w.next, w.pixmap, w.rowbits, C, H, W, h_out, w_out, pk,
                                                           ps, pp, policy, layout, bev_max_pix(C, pk, ps, kJC),
-                                                          bev_pairs_cap(C, pk, ps, kIB), out);
+                                                          bev_pairs_cap(C, pk, ps, kIB), out, w.argpos);
   LG_LAUNCH_OK();
   return LG_OK;
 }
@@ -614,24 +545,16 @@ extern "C" int lg_bev_backward(const int32_t* coords4, const float* feats, int64
   int rc = bev_check(n, C, batch_size, H, W, pk, ps, pp, policy, "lg_bev_backward");
   if (rc) return rc;
   const int64_t pixels = (int64_t)batch_size * H * W, rows = (int64_t)batch_size * C * H;
-  BevWorkspace w = carve_bev(const_cast<void*>(workspace), n, pixels, rows);
+  BevWorkspace w = carve_bev(const_cast<void*>(workspace), n, pixels, rows, bev_windows(batch_size, C, H, W, pk, ps, pp));
   LG_CHECK_ARG(workspace && workspace_bytes >= w.total, "lg_bev_backward: workspace too small");
   if (n == 0) return LG_OK;
   LG_CHECK_ARG(feats && grad_out && grad_feats, "lg_bev_backward: null pointer");
   const int h_out = (H + 2 * pp - pk) / ps + 1, w_out = (W + 2 * pp - pk) / ps + 1;
   LG_CHECK_ARG(layout == 0 || layout == 1, "lg_bev_backward: layout must be 0 (NCHW) or 1 (NHWC)");
-  LG_CUDA_OK(cudaMemsetAsync(grad_feats, 0, sizeof(float) * (size_t)n * C, stream));
-  const size_t smem = bev_smem_bwd(C, pk, ps);
-  const int64_t blocks = bev_tiles(batch_size, C, h_out, w_out, kJB);
-  LG_CHECK_ARG(blocks < ((int64_t)1 << 31), "lg_bev_backward: too many output tiles");
-  LG_CUDA_OK(cudaFuncSetAttribute(k_bev_pool_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_bev_pool_bwd<<<(unsigned)blocks, 256, smem, stream>>>(feats, w.next, w.pixmap, w.rowbits, C, H, W, h_out, w_out, pk,
-                                                          ps, pp, policy, layout, bev_max_pix(C, pk, ps, kJC),
-                                                          bev_pairs_cap(C, pk, ps, kIBh), grad_out, grad_feats);
+  const int64_t blocks = ceil_div(n, 8);  // a warp per voxel row
+  LG_CHECK_ARG(blocks < ((int64_t)1 << 31), "lg_bev_backward: too many rows");
+  k_bev_pool_bwd<<<(unsigned)blocks, 256, 0, stream>>>(feats, w.pix_of_row, w.next, w.pixmap, w.argpos, n, C, H, W,
+                                                       h_out, w_out, pk, ps, pp, policy, layout, grad_out, grad_feats);
   LG_LAUNCH_OK();
-  if (policy == LG_BEV_LAST) {
-    k_bev_dup_grad<<<(unsigned)ceil_div(n * C, 256), 256, 0, stream>>>(w.pix_of_row, w.pixmap, n, C, grad_feats);
-    LG_LAUNCH_OK();
-  }
   return LG_OK;
 }

@@ -39,7 +39,7 @@ class BevProjectFunction(torch.autograd.Function):
         w = (W + 2 * pp - pk) // ps + 1
         out = torch.empty((batch_size, C, h, w), dtype=torch.float32, device=feats.device,
                           memory_format=torch.channels_last if channels_last else torch.contiguous_format)
-        ws_bytes = L.lg_bev_workspace(n, C, batch_size, H, W)
+        ws_bytes = L.lg_bev_workspace(n, C, batch_size, H, W, pk, ps, pp)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=feats.device)
         cabi.check(L.lg_bev_forward(cabi.ptr(coords), cabi.ptr(feats_c), n, C, batch_size, float(bound),
                                     float(voxel_size), H, W, pk, ps, pp, policy, 1 if channels_last else 0,
