@@ -339,6 +339,23 @@ int lg_instnorm_backward(const float* dy, const float* x, const float* y, const 
                          int32_t B, const float* weight, int32_t relu, const double* stats, float* dx, float* dweight,
                          float* dbias, void* stream);
 
+/* ------------------------------------------------------------------ per-scan feature covariance (ISW loss)
+ *
+ * The statistic of RobustNet's instance-selective whitening loss, one of the baselines next to LiDOG (SURVEY.md 2.2):
+ * scan b = the rows whose batch index coords[r][0] is b (any row order), n_b of them, X_b their features (not centred).
+ *   cov float [B][C][C] = X_b^T X_b / (n_b - 1) + eps * I, exactly symmetric; eps * I when n_b <= 1;
+ *   counts int32 [B] = n_b, kept by the caller for the backward.
+ * 1 <= B <= 256 and 1 <= C <= 256 (LG_ERR_UNSUPPORTED outside), n < 2^31 - 1; rows with a batch index outside [0, B)
+ * are left out.  Features 16-byte aligned when C % 4 == 0.  Scratch: library arena.  Deterministic (fixed-order
+ * double merges, no float atomics). */
+int lg_inst_cov_forward(const float* x, const int32_t* coords, int64_t n, int32_t C, int32_t B, float eps, float* cov,
+                        int32_t* counts, void* stream);
+/* Backward: G float [B][C][C] = dL/dcov, counts from the forward;
+ * dx_r = x_r (G_b + G_b^T) / (n_b - 1) for the rows of scan b, 0 when n_b <= 1, NaN for rows outside [0, B).
+ * Every element of dx is written. */
+int lg_inst_cov_backward(const float* x, const int32_t* coords, int64_t n, int32_t C, int32_t B, const float* G,
+                         const int32_t* counts, float* dx, void* stream);
+
 /* ------------------------------------------------------------------ SyncBN exchange over peer memory
  *
  * train_lidog.py:228 converts every MinkowskiBatchNorm to SyncBN: 124 latency-bound exchanges of <= 3C doubles per

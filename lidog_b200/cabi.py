@@ -96,6 +96,8 @@ SIGNATURES = {
                                   _vp, _vp, _vp, _vp, _i32, _vp]),
     "lg_instnorm_forward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _f32, _i32, _vp, _vp, _i32, _vp, _vp]),
     "lg_instnorm_backward": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "lg_inst_cov_forward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _f32, _vp, _vp, _vp]),
+    "lg_inst_cov_backward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp]),
     "lg_peer_exchange_bytes": (_sz, []),
     "lg_peer_sum": (C.c_int, [_vp, _i32, C.POINTER(C.c_void_p), _i32, _i32, C.c_uint64, _vp, _vp]),
     "lg_dice_forward": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _f32, _i32, _vp, _vp, _vp]),
@@ -122,6 +124,7 @@ KERNELS_PER_CALL = {
     # + 1 (lg_prep_weights) when the call refreshes the 16-bit weights: counted by the caller
     "lg_conv_layer_infer": 1, "lg_confusion_matrix": 1,
     "lg_instnorm_forward": 3, "lg_instnorm_backward": 3,
+    "lg_inst_cov_forward": 5, "lg_inst_cov_backward": 2,
 }
 COUNTS: dict = {}
 _RAW = None

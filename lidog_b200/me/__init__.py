@@ -6,6 +6,7 @@ from .coords import CoordinateManager
 from .conv import MinkowskiConvolution, MinkowskiConvolutionTranspose, MinkowskiConvolutionBase, SparseConvFunction
 from .norm import (MinkowskiBatchNorm, MinkowskiSyncBatchNorm, MinkowskiInstanceNorm, MinkowskiReLU,
                    MinkowskiDropout)
+from .isw import instance_covariance, instance_whitening_loss
 from . import utils, modules
 
 __version__ = "0.5.4+lidog_b200"
