@@ -392,14 +392,17 @@ int lg_confusion_matrix(const float* logits, int64_t n, int32_t C, const int64_t
 /* ------------------------------------------------------------------ BEV projection */
 
 /* Bytes of the workspace that lg_bev_forward fills and lg_bev_backward reads, for the same arguments.  It holds the
- * pixel map, the row-occupancy words and the winning cell of every pooling window (one byte per output element:
- * ~340 MB at batch 8, C = 96, 2000 x 2000 -> 666 x 666). */
+ * pixel map, the row-occupancy words and the winning cell of every pooling window: one byte per output element,
+ * batch * C * h_out * w_out -- ~341 MB at batch 8, C = 96, 2000 x 2000 pooled 5/3/1 to 666 x 666, ~3.07 GB pooled
+ * 5/1/1 to 1998 x 1998. */
 size_t lg_bev_workspace(int64_t n, int32_t C, int32_t batch_size, int32_t H, int32_t W, int32_t pk, int32_t ps,
                         int32_t pp);
 
 /* Fused point-to-BEV projection: pixel scatter + raw (H,W,C)->(C,H,W) re-view + MaxPool2d(pk,ps,pp),
  * never materialising the dense tensor.  Replaces MinkUNetBaseBEV.sparse2super + filter_bounds
- * (utils/models/minkunet_bev.py:158-230).  out: float [batch, C, h, w], h = (H + 2pp - pk)/ps + 1, stored
+ * (utils/models/minkunet_bev.py:158-230).  Envelope: 1 <= pk <= 15, 1 <= ps <= 16, 0 <= 2 pp <= pk, h, w >= 1, any
+ * C >= 1, and batch*H*W, C*H*W, C*h*w < 2^31; anything else returns LG_ERR_INVALID before any CUDA call.
+ * out: float [batch, C, h, w], h = (H + 2pp - pk)/ps + 1 (12.3 GB at batch 8, C = 96, 1998 x 1998), stored
  * NCHW (layout 0) or NHWC / channels_last (layout 1: the same logical tensor, the memory order cuDNN's
  * tensor-op convolutions of the dense 2D head consume without staging copies).
  * workspace keeps the pixel map, the row-occupancy words and each window's winning cell for lg_bev_backward. */
@@ -407,10 +410,10 @@ int lg_bev_forward(const int32_t* coords4, const float* feats, int64_t n, int32_
                    float voxel_size, int32_t H, int32_t W, int32_t pk, int32_t ps, int32_t pp, int32_t policy,
                    int32_t layout, float* out, void* workspace, size_t workspace_bytes, void* stream);
 
-/* Backward of the above (autograd of index_put_ + max_pool2d at minkunet_bev.py:217-221).
+/* Backward of the above (autograd of index_put_ + max_pool2d at minkunet_bev.py:217-221); same envelope.
  * grad_feats [n, C] is fully written (rows outside the image get 0).  Atomic-free and bit-reproducible: every occupied
- * cell sums the <= 4 windows it won in ascending (i, j) order (the order of torch's CPU max_pool2d backward).
- * workspace: as the forward left it. */
+ * cell sums the <= ceil(pk/ps)^2 windows it won in ascending (i, j) order (the order of torch's CPU max_pool2d
+ * backward).  workspace: as the forward left it. */
 int lg_bev_backward(const int32_t* coords4, const float* feats, int64_t n, int32_t C, int32_t batch_size,
                     int32_t H, int32_t W, int32_t pk, int32_t ps, int32_t pp, int32_t policy, int32_t layout,
                     const float* grad_out, float* grad_feats, const void* workspace, size_t workspace_bytes,

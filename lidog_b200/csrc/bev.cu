@@ -17,9 +17,13 @@
 // coalesced loads per tile, only occupied rows touch the pixel map, only non-empty lines are scanned, and tiles move
 // as float4.  While it scans, the forward records the winning cell of every window that can hold a voxel in a
 // one-byte-per-window table (`argpos`).  The backward is one pass over the voxel rows, a warp per row and a lane per
-// channel: each (row, channel) cell adds up the <= 2 x 2 windows the table says it won, in ascending (i, j) order --
-// the order of torch's CPU max_pool2d backward, so the gradient is reproduced bit for bit -- and every element of the
-// gradient is written by exactly one thread: no atomics, no memset, run-to-run deterministic.
+// channel: each (row, channel) cell adds up the <= ceil(pk/ps)^2 windows the table says it won, in ascending (i, j)
+// order -- the order of torch's CPU max_pool2d backward, so the gradient is reproduced bit for bit -- and every element
+// of the gradient is written by exactly one thread: no atomics, no memset, run-to-run deterministic.
+// Geometry envelope (bev_check): 1 <= pk <= 15 (a window position fits the table's byte with 255 to spare),
+// 1 <= ps <= 16, 0 <= 2 pp <= pk, any C, H, W within int32 flat indices.  The tile height follows from ps so that a
+// tile's scrambled rows fit one 32-bit row mask, and images wider than 32 tile column blocks share one occupancy bit
+// between neighbouring blocks.
 #include "common.cuh"
 
 namespace lg {
@@ -28,7 +32,7 @@ struct BevWorkspace {
   int* pix_of_row;  // [n]      flat pixel (b*H*W + py*W + px) or -1
   int* next;        // [n]      chain of rows sharing a pixel (LG_BEV_MAX)
   int* pixmap;      // [B*H*W]  winner row (LAST) / chain head (MAX) / -1
-  uint32_t* rowbits;  // [B*C*H]  bit jt: scrambled row (c', h') holds a voxel inside tile column block jt
+  uint32_t* rowbits;  // [B*C*H]  bit jt >> grp_shift: scrambled row (c', h') holds a voxel inside tile column block jt
   unsigned char* argpos;  // [B*C*h_out*w_out] winning cell of a window ((h - h0) * pk + w - w0; 255 = an empty cell);
                           // written only for the (c', i) lines that can hold a voxel, which every voxel's window is on
   size_t total;
@@ -133,7 +137,8 @@ __device__ __forceinline__ int cell_argrow(int head, int ch, int C, int policy, 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Tiled pooling.  A CTA owns the output tile (b, 32 scrambled channels c', kIB rows i, kJC columns j).
+// Tiled pooling.  A CTA owns the output tile (b, 32 scrambled channels c', ib <= kIB rows i, kJC columns j); ib is the
+// largest height whose (ib - 1) * ps + pk scrambled rows fit the 32-bit row mask (bev_tile_rows).
 // Per (c', h') the cells of its windows are one contiguous run of <= (kJC-1)*ps+pk floats of the
 // never-materialised dense buffer, i.e. a handful of consecutive PIXELS, and only ~1-2 % of the pixels
 // hold a voxel.  Phase 1 reads one occupancy word per scrambled row (`rowbits`) and looks up the pixels of
@@ -143,7 +148,7 @@ __device__ __forceinline__ int cell_argrow(int head, int ch, int C, int policy, 
 // (channels_last, what cuDNN's tensor-op convolutions consume) or coalesced rows in NCHW.
 // No atomics; every output is written exactly once.
 constexpr int kCG = 32;   // scrambled channels per CTA
-constexpr int kIB = 8;    // output rows per CTA
+constexpr int kIB = 8;    // most output rows per CTA (collect_lines: 32 channels x 8 rows = 256 threads)
 constexpr int kJC = 32;   // output columns per CTA
 constexpr int kPitch = kCG + 4;  // floats per staged (i, j) cell group: float4-aligned, conflict-free 128-bit reads
 
@@ -152,7 +157,7 @@ struct TileGeom {
   int ncg, nib, njc;  // valid extents
   int h_lo, h_hi, w_lo, w_hi;  // cell region (clipped to the image), hi exclusive
   int jt;                      // tile column block
-  uint32_t jbits;              // rowbits bits that cover the cell columns of this geometry
+  uint32_t jbits;              // rowbits bit that covers the cell columns of this tile (block group jt >> grp_shift)
 };
 
 __device__ __forceinline__ void cell_region(TileGeom& g, int H, int W, int pk, int ps, int pp) {
@@ -162,21 +167,22 @@ __device__ __forceinline__ void cell_region(TileGeom& g, int H, int W, int pk, i
   g.w_hi = min((g.j0 + g.njc - 1) * ps - pp + pk, W);
 }
 
-__device__ __forceinline__ TileGeom tile_geom(int C, int H, int W, int h_out, int w_out, int pk, int ps, int pp) {
+__device__ __forceinline__ TileGeom tile_geom(int C, int H, int W, int h_out, int w_out, int pk, int ps, int pp, int ib,
+                                              int grp_shift) {
   TileGeom g;
-  const int n_jc = (w_out + kJC - 1) / kJC, n_ib = (h_out + kIB - 1) / kIB, n_cg = (C + kCG - 1) / kCG;
+  const int n_jc = (w_out + kJC - 1) / kJC, n_ib = (h_out + ib - 1) / ib, n_cg = (C + kCG - 1) / kCG;
   int idx = blockIdx.x;
   g.jt = idx % n_jc;
   g.j0 = g.jt * kJC;
   idx /= n_jc;
-  g.i0 = (idx % n_ib) * kIB;
+  g.i0 = (idx % n_ib) * ib;
   idx /= n_ib;
   g.c0 = (idx % n_cg) * kCG;
   g.b = idx / n_cg;
   g.ncg = min(kCG, C - g.c0);
-  g.nib = min(kIB, h_out - g.i0);
+  g.nib = min(ib, h_out - g.i0);
   g.njc = min(kJC, w_out - g.j0);
-  g.jbits = 1u << g.jt;
+  g.jbits = 1u << (g.jt >> grp_shift);
   cell_region(g, H, W, pk, ps, pp);
   return g;
 }
@@ -191,8 +197,8 @@ struct TileSmem {
 };
 
 // Phase 1.  Returns false (uniformly) when no pixel of the tile is occupied.  One coalesced rowbits load per
-// scrambled channel (lane = scrambled row, nrows <= 32 host-checked); only rows whose occupancy bit is set go to the
-// pixel map.
+// scrambled channel (lane = scrambled row; nrows <= 32 by the choice of the tile height); only rows whose occupancy bit
+// is set go to the pixel map.
 __device__ __forceinline__ bool tile_lookup(const TileGeom& g, const TileSmem& t, int C, int H, int W, int max_pix,
                                             const int* __restrict__ pixmap, const uint32_t* __restrict__ rowbits) {
   const int nrows = g.h_hi - g.h_lo;
@@ -250,7 +256,7 @@ __device__ __forceinline__ float window_scan(const TileGeom& g, const TileSmem& 
       ch -= C;
       ++d;
     }
-    for (int w = wa; w < wb;) {  // the <= pk cells of this row lie in one or two pixels: one head test per pixel
+    for (int w = wa; w < wb;) {  // the <= pk cells of this row lie in <= ceil(pk / C) + 1 pixels: one head test each
       const int span = min(wb - w, C - ch);
       const int head = t.heads[q * max_pix + d];
       if (head < 0) {  // a run of empty zeros; only its first cell can take the lead
@@ -347,11 +353,13 @@ __device__ __forceinline__ void collect_lines(const TileGeom& g, const TileSmem&
   __syncthreads();
 }
 
-__global__ void __launch_bounds__(256)
+// 4 blocks per SM: what the bench shape's ~51 KB of shared memory allows anyway; the register budget that follows
+// (64) keeps ptxas from spilling, which it did at its own choice of 48 registers
+__global__ void __launch_bounds__(256, 4)
     k_bev_pool_fwd(const float* __restrict__ feats, const int* __restrict__ next, const int* __restrict__ pixmap,
                    const uint32_t* __restrict__ rowbits, int C, int H, int W, int h_out, int w_out, int pk, int ps,
-                   int pp, int policy, int layout, int max_pix, int pairs_cap, float* __restrict__ out,
-                   unsigned char* __restrict__ argpos) {
+                   int pp, int policy, int layout, int ib, int grp_shift, int max_pix, int pairs_cap,
+                   float* __restrict__ out, unsigned char* __restrict__ argpos) {
   extern __shared__ __align__(16) unsigned char s_dyn[];
   TileSmem t;
   t.out = reinterpret_cast<float*>(s_dyn);
@@ -360,7 +368,7 @@ __global__ void __launch_bounds__(256)
   t.rowmask = reinterpret_cast<uint32_t*>(t.plo + pairs_cap);
   t.n_lines = reinterpret_cast<int*>(t.rowmask + kCG);
   t.lines = reinterpret_cast<unsigned short*>(t.n_lines + 1);
-  const TileGeom g = tile_geom(C, H, W, h_out, w_out, pk, ps, pp);
+  const TileGeom g = tile_geom(C, H, W, h_out, w_out, pk, ps, pp, ib, grp_shift);
   {  // zero the staged tile: most lines pool zeros only and are never touched again
     float4* o4 = reinterpret_cast<float4*>(t.out);
     const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -389,11 +397,16 @@ __global__ void __launch_bounds__(256)
 
 // Backward.  The gradient of a window goes to its first arg-max in scan order (max_pool2d backward) if that cell
 // holds a voxel; the forward left the cell's position in `argpos`.  A warp owns one voxel row, lane = channel, so the
-// row's writes are coalesced.  The row's cell (c', h, w) sits in <= 2 x 2 windows (host-checked: pk <= 2 ps) and adds
-// up those whose table entry names it in ascending (i, j) order -- the order of torch's CPU max_pool2d backward, so
-// the gradient is bit-equal to it.  LAST: every row of the pixel computes the same sum (index_put_ backward hands the
-// pixel's gradient to each row that wrote it); MAX: only the chain's first row attaining the cell's max receives it.
-// Every element of grad_feats is written exactly once, rows outside the image with 0: no memset, no atomics.
+// row's writes are coalesced.  The row's cell (c', h, w) sits in the windows i in [ceil((h + pp - pk + 1) / ps),
+// floor((h + pp) / ps)] (clipped to the output), likewise for j, and adds up those whose table entry names it in
+// ascending (i, j) order -- the order of torch's CPU max_pool2d backward, so the gradient is bit-equal to it.
+// LAST: every row of the pixel computes the same sum (index_put_ backward hands the pixel's gradient to each row that
+// wrote it); MAX: only the chain's first row attaining the cell's max receives it.  Every element of grad_feats is
+// written exactly once, rows outside the image with 0: no memset, no atomics.
+// The pass is latency-bound (each row waits on its pixel, then its table bytes, then its gradient reads), so loads
+// are issued in groups.  WIDE = false (pk <= 2 ps: at most 2 x 2 windows per cell): kU channels' windows unrolled
+// together.  WIDE = true (up to 15 x 15 windows): one channel at a time, its windows in groups of kG.
+template <bool WIDE>
 __global__ void __launch_bounds__(256)
     k_bev_pool_bwd(const float* __restrict__ feats, const int* __restrict__ pix_of_row, const int* __restrict__ next,
                    const int* __restrict__ pixmap, const unsigned char* __restrict__ argpos, int64_t n, int C, int H,
@@ -414,45 +427,79 @@ __global__ void __launch_bounds__(256)
   const int64_t sample = (int64_t)b * C * h_out * w_out;  // C * h_out * w_out < 2^31 (host-checked)
   const unsigned char* tab = argpos + sample;
   const float* go = grad_out + sample;
-  // kU channels per lane at a time, unrolled, so that their table reads and then their gradient reads are in flight
-  // together: one channel at a time left a chain of dependent loads per channel and the pass latency-bound (0.77 ms
-  // at the bench shape).  3 takes the bench's 96 channels in one pass (0.64 ms); 4 needs 68 registers, keeps fewer
-  // warps resident and measured 0.80 ms (profiles/r05_bev_bench.jsonl).
-  constexpr int kU = 3;
-  for (int base = lane; base < C; base += 32 * kU) {
-    bool hit[kU][4];
-    int off[kU][4];
+  if constexpr (!WIDE) {
+    // kU channels per lane at a time, unrolled, so that their table reads and then their gradient reads are in flight
+    // together: one channel at a time left a chain of dependent loads per channel (0.77 ms at the bench shape).  3 takes
+    // the bench's 96 channels in one pass (0.64 ms); 4 needs 68 registers, keeps fewer warps resident and measured
+    // 0.80 ms (profiles/r05_bev_bench.jsonl).
+    constexpr int kU = 3;
+    for (int base = lane; base < C; base += 32 * kU) {
+      bool hit[kU][4];
+      int off[kU][4];
 #pragma unroll
-    for (int k = 0; k < kU; ++k) {
-      const int ch = base + 32 * k;
+      for (int k = 0; k < kU; ++k) {
+        const int ch = base + 32 * k;
 #pragma unroll
-      for (int q = 0; q < 4; ++q) hit[k][q] = false, off[k][q] = 0;
-      if (ch < C && (policy == LG_BEV_LAST || cell_argrow(head, ch, C, policy, feats, next) == (int)r)) {
-        // scrambled cell (c', h, w): the (H, W, C) buffer re-viewed as (C, H, W); m < C * H * W < 2^31 (host-checked)
-        const int m = m0 + ch, c = m / hw, h = (m - c * hw) / W, w = m - c * hw - h * W;
-        // window rows containing h: qi - 1 (h at row offset ri + ps) and qi (offset ri), where it lies inside them
-        const int qi = (unsigned)(h + pp) / (unsigned)ps, ri = h + pp - qi * ps;
-        const int qj = (unsigned)(w + pp) / (unsigned)ps, rj = w + pp - qj * ps;
+        for (int q = 0; q < 4; ++q) hit[k][q] = false, off[k][q] = 0;
+        if (ch < C && (policy == LG_BEV_LAST || cell_argrow(head, ch, C, policy, feats, next) == (int)r)) {
+          // scrambled cell (c', h, w): the (H, W, C) buffer re-viewed as (C, H, W); m < C * H * W < 2^31 (host-checked)
+          const int m = m0 + ch, c = m / hw, h = (m - c * hw) / W, w = m - c * hw - h * W;
+          // window rows containing h: qi - 1 (h at row offset ri + ps) and qi (offset ri), where it lies inside them
+          const int qi = (unsigned)(h + pp) / (unsigned)ps, ri = h + pp - qi * ps;
+          const int qj = (unsigned)(w + pp) / (unsigned)ps, rj = w + pp - qj * ps;
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {  // ascending (i, j)
-          const int di = 1 - (q >> 1), dj = 1 - (q & 1);
-          const int i = qi - di, j = qj - dj, oh = ri + di * ps, ow = rj + dj * ps;
-          if (i >= 0 && i < h_out && oh < pk && j >= 0 && j < w_out && ow < pk) {
-            const int t = (c * h_out + i) * w_out + j;
-            hit[k][q] = __ldg(tab + t) == oh * pk + ow;
-            off[k][q] = layout ? (i * w_out + j) * C + c : t;
+          for (int q = 0; q < 4; ++q) {  // ascending (i, j)
+            const int di = 1 - (q >> 1), dj = 1 - (q & 1);
+            const int i = qi - di, j = qj - dj, oh = ri + di * ps, ow = rj + dj * ps;
+            if (i >= 0 && i < h_out && oh < pk && j >= 0 && j < w_out && ow < pk) {
+              const int t = (c * h_out + i) * w_out + j;
+              hit[k][q] = __ldg(tab + t) == oh * pk + ow;
+              off[k][q] = layout ? (i * w_out + j) * C + c : t;
+            }
           }
         }
       }
+#pragma unroll
+      for (int k = 0; k < kU; ++k) {
+        const int ch = base + 32 * k;
+        float sum = 0.f;
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+          if (hit[k][q]) sum += __ldg(go + off[k][q]);
+        if (ch < C) gf[ch] = sum;
+      }
     }
-#pragma unroll
-    for (int k = 0; k < kU; ++k) {
-      const int ch = base + 32 * k;
+  } else {
+    // the cell's ni x nj windows, flattened in ascending (i, j) order, kG at a time: their table bytes, then the
+    // gradients of the hits, are in flight together
+    constexpr int kG = 8;
+    for (int ch = lane; ch < C; ch += 32) {
       float sum = 0.f;
+      if (policy == LG_BEV_LAST || cell_argrow(head, ch, C, policy, feats, next) == (int)r) {
+        const int m = m0 + ch, c = m / hw, h = (m - c * hw) / W, w = m - c * hw - h * W;
+        const int i_lo = max(h + pp - pk + 1 + ps - 1, 0) / ps, i_hi = min((h + pp) / ps, h_out - 1);
+        const int j_lo = max(w + pp - pk + 1 + ps - 1, 0) / ps, j_hi = min((w + pp) / ps, w_out - 1);
+        const int nj = j_hi - j_lo + 1, nwin = i_lo <= i_hi && j_lo <= j_hi ? (i_hi - i_lo + 1) * nj : 0;
+        for (int t0 = 0; t0 < nwin; t0 += kG) {
+          bool hit[kG];
+          int off[kG];
 #pragma unroll
-      for (int q = 0; q < 4; ++q)
-        if (hit[k][q]) sum += __ldg(go + off[k][q]);
-      if (ch < C) gf[ch] = sum;
+          for (int k = 0; k < kG; ++k) {
+            hit[k] = false;
+            off[k] = 0;
+            if (t0 + k < nwin) {
+              const int i = i_lo + (t0 + k) / nj, j = j_lo + (t0 + k) % nj;
+              const int t = (c * h_out + i) * w_out + j;
+              hit[k] = __ldg(tab + t) == (h + pp - i * ps) * pk + (w + pp - j * ps);
+              off[k] = layout ? (i * w_out + j) * C + c : t;
+            }
+          }
+#pragma unroll
+          for (int k = 0; k < kG; ++k)
+            if (hit[k]) sum += __ldg(go + off[k]);
+        }
+      }
+      gf[ch] = sum;
     }
   }
 }
@@ -461,36 +508,45 @@ __global__ void __launch_bounds__(256)
 
 using namespace lg;
 
+// output rows per tile: the tile's (ib - 1) * ps + pk scrambled rows must fit the 32-bit row mask (>= 1 as pk <= 15)
+static int bev_tile_rows(int pk, int ps) { const int r = (32 - pk) / ps + 1; return r < kIB ? r : kIB; }
+// log2 of the tile column blocks per occupancy bit: a row's one 32-bit word covers images wider than 32 blocks
+static int bev_col_shift(int w_out) {
+  int s = 0;
+  while ((32 << s) < ceil_div(w_out, kJC)) ++s;
+  return s;
+}
 // a (c', h') run of a tile spans (cols-1)*ps+pk floats = at most this many pixels of C channels
 static int bev_max_pix(int C, int pk, int ps, int cols) { return ((cols - 1) * ps + pk + C - 2) / C + 1; }
 static int bev_pairs_cap(int C, int pk, int ps, int rows) { return (C < kCG ? C : kCG) * ((rows - 1) * ps + pk); }
 static size_t bev_smem_fwd(int C, int pk, int ps) {  // staged tile + heads + first pixels + row masks
-  const size_t pairs = bev_pairs_cap(C, pk, ps, kIB);
+  const size_t pairs = bev_pairs_cap(C, pk, ps, bev_tile_rows(pk, ps));
   return sizeof(float) * kIB * kJC * kPitch + sizeof(int) * pairs * (bev_max_pix(C, pk, ps, kJC) + 1) + sizeof(int) * kCG +
          sizeof(int) + 2 * kCG * kIB + 16;
 }
-static int64_t bev_tiles(int B, int C, int h_out, int w_out) {
-  return (int64_t)B * ceil_div(C, kCG) * ceil_div(h_out, kIB) * ceil_div(w_out, kJC);
+static int64_t bev_tiles(int B, int C, int h_out, int w_out, int ib) {
+  return (int64_t)B * ceil_div(C, kCG) * ceil_div(h_out, ib) * ceil_div(w_out, kJC);
 }
 // pooling windows of the output (entries of the argpos table); 0 for parameters bev_check rejects
 static int64_t bev_windows(int B, int C, int H, int W, int pk, int ps, int pp) {
-  if (B < 1 || C < 1 || ps < 1) return 0;
+  if (B < 1 || C < 1 || ps < 1 || H + 2 * pp < pk || W + 2 * pp < pk) return 0;
   const int64_t h_out = (H + 2 * pp - pk) / ps + 1, w_out = (W + 2 * pp - pk) / ps + 1;
-  return h_out > 0 && w_out > 0 ? (int64_t)B * C * h_out * w_out : 0;
+  return (int64_t)B * C * h_out * w_out;
 }
 
 static int bev_check(int64_t n, int C, int B, int H, int W, int pk, int ps, int pp, int policy, const char* who) {
   LG_CHECK_ARG(n >= 0 && C >= 1 && B >= 1 && H >= 1 && W >= 1, "%s: bad sizes", who);
-  LG_CHECK_ARG(pk >= 1 && ps >= 1 && pp >= 0 && 2 * pp <= pk, "%s: bad pooling parameters", who);
+  LG_CHECK_ARG(pk >= 1 && pk <= 15, "%s: pool kernel %d outside 1..15 (the one-byte argpos table)", who, pk);
+  LG_CHECK_ARG(ps >= 1 && ps <= 16, "%s: pool stride %d outside 1..16", who, ps);
+  LG_CHECK_ARG(pp >= 0 && 2 * pp <= pk, "%s: pool padding %d outside 0..pk/2", who, pp);
+  LG_CHECK_ARG(H + 2 * pp >= pk && W + 2 * pp >= pk, "%s: image smaller than the pool window (h_out, w_out < 1)", who);
   LG_CHECK_ARG(policy == LG_BEV_LAST || policy == LG_BEV_MAX, "%s: bad policy", who);
   LG_CHECK_ARG((int64_t)B * H * W < ((int64_t)1 << 31), "%s: batch*H*W exceeds int32", who);
-  LG_CHECK_ARG(kIB * ps + pk <= 32, "%s: pool stride/kernel too large for the row mask", who);
-  LG_CHECK_ARG(pk <= 2 * ps && pk * pk < 255, "%s: a cell may sit in at most 2 x 2 windows (pk <= 2 ps)", who);
   LG_CHECK_ARG((int64_t)C * H * W < ((int64_t)1 << 31), "%s: C*H*W exceeds int32", who);
   const int h_out = (H + 2 * pp - pk) / ps + 1, w_out = (W + 2 * pp - pk) / ps + 1;
   LG_CHECK_ARG((int64_t)C * h_out * w_out < ((int64_t)1 << 31), "%s: C*h_out*w_out exceeds int32", who);
-  LG_CHECK_ARG(ceil_div(w_out, kJC) <= 32, "%s: more than 32 tile column blocks (W too large for the occupancy word)", who);
-  LG_CHECK_ARG(bev_smem_fwd(C, pk, ps) <= 200 * 1024, "%s: C=%d too small for pool stride %d (shared memory)", who, C, ps);
+  // never fires inside the envelope above (at most 108 KB, at C = 31, pk = 15, ps = 16); guards the launch below
+  LG_CHECK_ARG(bev_smem_fwd(C, pk, ps) <= 200 * 1024, "%s: forward tile needs more than 200 KB of shared memory", who);
   return LG_OK;
 }
 
@@ -514,6 +570,7 @@ extern "C" int lg_bev_forward(const int32_t* coords4, const float* feats, int64_
   LG_CHECK_ARG(layout == 0 || layout == 1, "lg_bev_forward: layout must be 0 (NCHW) or 1 (NHWC)");
   LG_CHECK_ARG(((uintptr_t)out & 15) == 0, "lg_bev_forward: out must be 16-byte aligned");
   const int h_out = (H + 2 * pp - pk) / ps + 1, w_out = (W + 2 * pp - pk) / ps + 1;
+  const int ib = bev_tile_rows(pk, ps), grp_shift = bev_col_shift(w_out), grp = 1 << grp_shift;
   LG_CUDA_OK(cudaMemsetAsync(w.pixmap, 0xFF, sizeof(int) * (size_t)pixels, stream));
   LG_CUDA_OK(cudaMemsetAsync(w.rowbits, 0, sizeof(uint32_t) * (size_t)rows, stream));
   if (n > 0) {
@@ -521,18 +578,20 @@ extern "C" int lg_bev_forward(const int32_t* coords4, const float* feats, int64_
                                                                  voxel_size, H, W, policy, w.pix_of_row, w.next,
                                                                  w.pixmap);
     LG_LAUNCH_OK();
-    k_bev_rowbits<<<(unsigned)ceil_div(n, 256), 256, 0, stream>>>(w.pix_of_row, n, C, H, W, kJC * ps,
-                                                                  (kJC - 1) * ps + pk, pp, (int)ceil_div(w_out, kJC),
-                                                                  w.rowbits);
+    // an occupancy bit stands for grp neighbouring tile column blocks
+    k_bev_rowbits<<<(unsigned)ceil_div(n, 256), 256, 0, stream>>>(w.pix_of_row, n, C, H, W, grp * kJC * ps,
+                                                                  (grp * kJC - 1) * ps + pk, pp,
+                                                                  (int)ceil_div(ceil_div(w_out, kJC), grp), w.rowbits);
     LG_LAUNCH_OK();
   }
   const size_t smem = bev_smem_fwd(C, pk, ps);
-  const int64_t blocks = bev_tiles(batch_size, C, h_out, w_out);
+  const int64_t blocks = bev_tiles(batch_size, C, h_out, w_out, ib);
   LG_CHECK_ARG(blocks < ((int64_t)1 << 31), "lg_bev_forward: too many output tiles");
   LG_CUDA_OK(cudaFuncSetAttribute(k_bev_pool_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k_bev_pool_fwd<<<(unsigned)blocks, 256, smem, stream>>>(feats, w.next, w.pixmap, w.rowbits, C, H, W, h_out, w_out, pk,
-                                                          ps, pp, policy, layout, bev_max_pix(C, pk, ps, kJC),
-                                                          bev_pairs_cap(C, pk, ps, kIB), out, w.argpos);
+                                                          ps, pp, policy, layout, ib, grp_shift,
+                                                          bev_max_pix(C, pk, ps, kJC), bev_pairs_cap(C, pk, ps, ib), out,
+                                                          w.argpos);
   LG_LAUNCH_OK();
   return LG_OK;
 }
@@ -553,8 +612,10 @@ extern "C" int lg_bev_backward(const int32_t* coords4, const float* feats, int64
   LG_CHECK_ARG(layout == 0 || layout == 1, "lg_bev_backward: layout must be 0 (NCHW) or 1 (NHWC)");
   const int64_t blocks = ceil_div(n, 8);  // a warp per voxel row
   LG_CHECK_ARG(blocks < ((int64_t)1 << 31), "lg_bev_backward: too many rows");
-  k_bev_pool_bwd<<<(unsigned)blocks, 256, 0, stream>>>(feats, w.pix_of_row, w.next, w.pixmap, w.argpos, n, C, H, W,
-                                                       h_out, w_out, pk, ps, pp, policy, layout, grad_out, grad_feats);
+  // pk <= 2 ps: a cell lies in at most 2 x 2 windows, which the unrolled variant takes in one go
+  auto kernel = pk <= 2 * ps ? k_bev_pool_bwd<false> : k_bev_pool_bwd<true>;
+  kernel<<<(unsigned)blocks, 256, 0, stream>>>(feats, w.pix_of_row, w.next, w.pixmap, w.argpos, n, C, H, W, h_out, w_out,
+                                               pk, ps, pp, policy, layout, grad_out, grad_feats);
   LG_LAUNCH_OK();
   return LG_OK;
 }

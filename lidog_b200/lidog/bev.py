@@ -26,6 +26,22 @@ def image_size(bound: float, voxel_size: float) -> int:
     return int(torch.tensor((bound - (-bound)) / voxel_size).int())
 
 
+def pool_for_scaling(scaling_factor: float = 1.0) -> tuple:
+    """MaxPool2d (kernel, stride, padding) of the reference's `sparse2super(x, input_voxel_size, scaling_factor)`
+    (minkunet_bev.py:151-156, 222-224): stride 3 at s = 1, else int(3 / s).  The fused operator takes strides 1..16."""
+    return (5, 3, 1) if scaling_factor == 1.0 else (5, int(3 / scaling_factor), 1)
+
+
+def label_image_size(bound: float, voxel_size: float, pool=(5, 3, 1)) -> int:
+    """Side of the BEV label image: the output of `Encoder2D` (two stride-2 3x3 convolutions, each ceil(h / 2)) on the
+    pooled projection.  167 for the KITTI bound of 50 m and 100 for nuScenes' 30 m, at voxel 0.05 and pool 5/3/1."""
+    pk, ps, pp = pool
+    h = (image_size(bound, voxel_size) + 2 * pp - pk) // ps + 1
+    for _ in range(2):
+        h = (h + 1) // 2
+    return h
+
+
 class BevProjectFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, feats, coords, batch_size, bound, voxel_size, pool, policy, channels_last):
@@ -85,9 +101,8 @@ def patch_reference_model(model, policy="last"):
     """Route an instance of the reference's MinkUNetBaseBEV (unchanged class) to the fused operator."""
 
     def _s2s(self, x, input_voxel_size=0.05, scaling_factor=1.0):
-        stride = 3 if scaling_factor == 1.0 else int(3 / scaling_factor)
-        return sparse2super(x, bound=self.mapping_bound_2d, voxel_size=input_voxel_size, pool=(5, stride, 1),
-                            policy=policy)
+        return sparse2super(x, bound=self.mapping_bound_2d, voxel_size=input_voxel_size,
+                            pool=pool_for_scaling(scaling_factor), policy=policy)
 
     model.sparse2super = types.MethodType(_s2s, model)
 

@@ -73,8 +73,10 @@ class Encoder2D(nn.Module):
 
 class MinkUNet34BEV(nn.Module):
     def __init__(self, in_channels, out_channels, D=3, initial_kernel_size=5, decoder_2d_level=("block8",),
-                 mapping_bound_2d=50.0, ME=None, bev_fn=None, bev_policy="last", layers=LAYERS34):
+                 mapping_bound_2d=50.0, ME=None, bev_fn=None, bev_policy="last", layers=LAYERS34,
+                 bev_scaling_factor=1.0):
         super().__init__()
+        from lidog_b200.lidog.bev import pool_for_scaling
         if ME is None:
             from lidog_b200 import me as ME
         if bev_fn is None:
@@ -82,6 +84,9 @@ class MinkUNet34BEV(nn.Module):
         self._ME, self._bev_fn, self.bev_policy = ME, bev_fn, bev_policy
         self.D = D
         self.mapping_bound_2d = mapping_bound_2d
+        # the reference's sparse2super scaling factor as a MaxPool2d (kernel, stride, padding); no parameters depend
+        # on it, so the state dict is the same at every factor
+        self.bev_pool = pool_for_scaling(bev_scaling_factor)
         self.decoder_2d_level = list(decoder_2d_level)
         Block = ME.modules.resnet_block.BasicBlock
         conv, convtr, bn = ME.MinkowskiConvolution, ME.MinkowskiConvolutionTranspose, ME.MinkowskiBatchNorm
@@ -131,7 +136,7 @@ class MinkUNet34BEV(nn.Module):
                 nn.init.constant_(m.bn.bias, 0)
 
     def sparse2super(self, x, input_voxel_size=0.05):
-        return self._bev_fn(x, bound=self.mapping_bound_2d, voxel_size=input_voxel_size, pool=(5, 3, 1),
+        return self._bev_fn(x, bound=self.mapping_bound_2d, voxel_size=input_voxel_size, pool=self.bev_pool,
                             policy=self.bev_policy)
 
     def forward(self, x, is_seg=True, is_train=False):

@@ -16,6 +16,7 @@ import os
 import torch
 
 from . import losses
+from .bev import label_image_size
 from .synth import SHAPES
 
 
@@ -65,7 +66,10 @@ class LidogTrainer:
         self.buffer_sync = buffer_sync  # lidog/ddp.py FlatBuffers: rank 0's BN buffers broadcast at the start of a step
         self.num_classes, self.voxel_size, self.ignore_label = num_classes, voxel_size, ignore_label
         self.source_weights = source_weights
-        self.bound, self.bev_img = SHAPES[shape]["bound"], SHAPES[shape]["bev_img"]
+        # the label image has the size of the BEV head's output at the model's pooling (SHAPES' bev_img at the default)
+        pool = getattr(getattr(model, "module", model), "bev_pool", (5, 3, 1))
+        self.bound = SHAPES[shape]["bound"]
+        self.bev_img = label_image_size(self.bound, voxel_size, pool)
         params = list(model.parameters())
         # same update rule as the reference's torch.optim.Adam (trainer_lighting_2d.py:349-360); on the GPU the
         # ~190 parameter tensors are updated by the fused multi-tensor kernels instead of one launch per op
